@@ -9,8 +9,14 @@ Modes = the BASELINE.json configs (default: lz4-compress, the config the headlin
     lz4-decompress  configs[2]  lz4-mt decompress-only, 32 GiB stream framed by the REFERENCE, 1->8 GPUs  (strong scaling)
     zstd-compress   configs[3]  zstd-mt level 3, 8 GiB synthetic text per GPU, 1 MiB chunks              (weak scaling)
     zstd-mix        configs[4]  zstd-mt level 3, Silesia-mix, 4 MiB chunks, 8 GiB per GPU (64 GiB at 8)  (weak scaling)
-The default run also carries short device-timed legs of the other configs in `extra` (so the driver's 1->8 sweep
-records them at every N); `--no-extra` drops them.
+The default run also carries short device-timed legs of the other configs in `extra` (so a 1->8 GPU sweep records
+them at every N); `--no-extra` drops them.  `--steps K` is the number of timed steps of every device-timed leg.
+
+--dump-outputs DIR writes what the timed path computed in its last step, as float32 / float64 .npy files (rank 0's
+share under N>1), so that two builds can be compared output for output on identical inputs:
+    compress modes  : frame_offsets (the frame_off array, all of it), framed_sample_positions + framed_sample (a fixed,
+                      seeded sample of the framed bytes)
+    lz4-decompress  : status and out_size (per frame, all of them), decoded_sample_positions + decoded_sample
 
 A step = one pass of the per-chunk hot path over the whole batch:
   value    : GB/s of (bytes in + bytes out), device-timed with CUDA events, inputs resident in HBM, max over ranks
@@ -37,6 +43,8 @@ import numpy as np
 
 GIB = 1 << 30
 DEAL_BATCH = 8            # chunks per dealt batch (host_api.cpp: compress slots hold 8 MiB = 8 chunks of 1 MiB)
+DUMP_SAMPLES = 1 << 21    # sampled bytes per --dump-outputs buffer: 8 B position + 4 B value each, 24 MiB
+DUMP_SEED = 20240601
 
 MODES = {
     "lz4-compress": dict(codec="lz4", op="c", kind="mix", chunk_mib=1, gib=8.0, level=1, scaling="weak",
@@ -72,6 +80,7 @@ def parse_args():
     ap.add_argument("--no-extra", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="device-timed leg only (profiling runs under ncu)")
     ap.add_argument("--no-bind", action="store_true", help="do not bind the rank's process to the CPUs next to its GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the last timed step's outputs to DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -177,15 +186,13 @@ def ref_fn(o, codec, op):
     return getattr(o.ref(), "ref_%s_%s_mem" % (codec, "compress" if op == "c" else "decompress"))
 
 
-def ref_framed_segment(z, o, M, seg_bytes, threads):
-    """A Silesia-mix segment framed by the UNMODIFIED reference (LZ4MT/ZSTDCB_compressCCtx on the host cores)."""
+def ref_framed_segment(z, o, M, seg_bytes):
+    """A Silesia-mix segment framed as the UNMODIFIED reference frames it (LZ4MT/ZSTDCB_compressCCtx): the same
+    liblz4 / libzstd call per chunk behind the same 12-byte headers, byte for byte (tests/_oracle.py lib_compress,
+    checked against digests of the reference's output by the test suite)."""
     chunk = M["chunk_mib"] << 20
     src = z.gen_stream(kind_id(z, M["kind"]), seg_bytes, chunk)
-    cap = seg_bytes + seg_bytes // 64 + (1 << 20)
-    out = np.empty(cap, np.uint8); st = (ctypes.c_size_t * 5)()
-    rc = ref_fn(o, M["codec"], "c")(threads, M["level"], chunk, src.ctypes.data, seg_bytes, out.ctypes.data, cap, st)
-    assert rc == 0, "reference compress failed: %d" % rc
-    return src, out[: int(st[0])].copy()
+    return src, o.lib_compress(o.CODEC_LZ4 if M["codec"] == "lz4" else o.CODEC_ZSTD, src, M["level"], chunk)
 
 
 # =============================================================================== reference arm
@@ -218,7 +225,7 @@ def run_reference(args):
         sample = "first %d MiB of the workload per step, %s_compressCCtx(T=%d, level %d, %d MiB chunks), memory-to-memory callbacks" % (
             n >> 20, "LZ4MT" if M["codec"] == "lz4" else "ZSTDCB", threads, M["level"], M["chunk_mib"])
     else:
-        src, framed = ref_framed_segment(z, o, M, n, threads)
+        src, framed = ref_framed_segment(z, o, M, n)
         back = np.empty(n + 16, np.uint8)
         fn = ref_fn(o, M["codec"], "d")
         def step():
@@ -333,6 +340,17 @@ def timed_steps(job, L, fn, steps, warmup):
     return job.reduce(mine, "max"), mine, [ms[i] / max(cnt[i], 1) for i in range(16)], [int(cnt[i]) for i in range(16)], clocks
 
 
+def sample_device_bytes(torch, buf, nbytes, prefix):
+    """A fixed, seeded sample of the first `nbytes` of a device byte buffer: {prefix_positions: float64, prefix: float32}.
+    The positions depend on nbytes and DUMP_SEED only, so equal-length outputs are sampled at the same places."""
+    if nbytes <= DUMP_SAMPLES:
+        pos = np.arange(nbytes, dtype=np.int64)
+    else:
+        pos = np.sort(np.random.default_rng(DUMP_SEED).integers(0, nbytes, DUMP_SAMPLES, dtype=np.int64))
+    vals = buf[torch.from_numpy(pos).to(buf.device)].cpu().numpy()
+    return {prefix + "_positions": pos.astype(np.float64), prefix: vals.astype(np.float32)}
+
+
 def roofline(kms, algorithmic_bytes, ids):
     """The dominant kernel among `ids` (largest mean launch time) against the measured HBM peak."""
     peak, peak_src = measured_peaks()
@@ -391,6 +409,10 @@ def leg_compress(job, args, M, gib, steps, warmup, full):
     comp = (z.Lz4DeviceCompressor if lz4 else z.ZstdDeviceCompressor)(n, chunk)
     dev_ms, my_ms, kms, cnt, clocks = timed_steps(job, L, lambda: comp.run(d_in, job.stream), steps, warmup)
     framed = int(comp.frame_off[-1].item())
+    outputs = None
+    if full and args.dump_outputs:                      # (out, frame_off) of the last timed step
+        outputs = {"frame_offsets": comp.frame_off.cpu().numpy().astype(np.float64)}
+        outputs.update(sample_device_bytes(torch, comp.out, framed, "framed_sample"))
     alg_mine = n + framed
     total_alg = job.reduce(alg_mine, "sum")
     ids = [0, 1, 2, 3, 4] if lz4 else [7, 8]
@@ -398,7 +420,7 @@ def leg_compress(job, args, M, gib, steps, warmup, full):
            "per_rank_ms": [x / steps for x in job.gather(my_ms)], "per_rank_kernel_ms": job.gather(kms[ids[0]]),
            "kernel_ms": {KERNEL_NAMES[i]: kms[i] for i in ids}, "launches": int(job.reduce((5 if lz4 else 4) * steps, "sum")),      # kernels per step: lz4 5 (all event-timed), zstd 4
            "roofline": roofline(kms, alg_mine, ids[:1]), "clocks": clocks, "gen_seconds": gen_s,
-           "n": n, "chunk": chunk, "nchunks": nchunks, "framed": framed, "alg_mine": alg_mine}
+           "n": n, "chunk": chunk, "nchunks": nchunks, "framed": framed, "alg_mine": alg_mine, "outputs": outputs}
     # ---- parity gate at full size (not timed): GPU decode of the GPU stream == the input, on the device
     out, foff = comp.out, comp.frame_off
     if lz4:
@@ -524,9 +546,9 @@ def cpu_baseline(args, M, src, n, chunk, codec_fn_c, codec_fn_d, with_decode):
 
 
 # ------------------------------------------------------------------------------- decompress leg (configs[2])
-def leg_lz4_decompress(job, args, M, total_gib, steps, warmup, seg_gib=2.0):
+def leg_lz4_decompress(job, args, M, total_gib, steps, warmup, seg_gib=2.0, dump=False):
     """Device-timed decode of a stream framed by the reference: a `seg_gib` framed segment tiled to `total_gib`, tiles
-    dealt round-robin over the ranks (strong scaling).  Falls back to a GPU-framed segment when oracle/_ref is absent."""
+    dealt round-robin over the ranks (strong scaling)."""
     import zstdmt_b200 as z
     torch = job.torch
     L = z.lib()
@@ -535,17 +557,9 @@ def leg_lz4_decompress(job, args, M, total_gib, steps, warmup, seg_gib=2.0):
     seg = min(int(seg_gib * GIB), total) // chunk * chunk
     tiles = max(1, total // seg)
     mine = [t for t in range(tiles) if t % job.world == job.rank]
-    T = min(os.cpu_count() or 1, 128)
-    framer = "reference (LZ4MT_compressCCtx level 1, liblz4 1.9.4, linked blocks)"
-    try:
-        import _oracle as o
-        assert o.have_ref()
-        src, framed = ref_framed_segment(z, o, M, seg, max(8, T // max(job.world, 1)))
-    except Exception as e:
-        framer = "GPU encoder (independent blocks) — oracle/_ref unavailable: %r" % (e,)
-        src = z.gen_stream(kind_id(z, M["kind"]), seg, chunk)
-        rc, framed, _ = z.compress_mem(z.CODEC_LZ4, src, threads=4, level=1, chunk=chunk)
-        assert rc == 0
+    import _oracle as o
+    src, framed = ref_framed_segment(z, o, M, seg)
+    framer = "reference framing (LZ4MT_compressCCtx level 1 layout, liblz4 %s, linked blocks)" % o.library_versions()["liblz4"]
     offs, sizes = z.scan_frames(framed)
     nf = len(offs)
     k = max(1, len(mine))
@@ -566,6 +580,10 @@ def leg_lz4_decompress(job, args, M, total_gib, steps, warmup, seg_gib=2.0):
     for i in range(k):
         assert torch.equal(dout[i * seg:(i + 1) * seg], d_src), "decode of the reference-framed stream differs from the source (tile %d)" % i
     dev_ms, my_ms, kms, cnt, clocks = timed_steps(job, L, run, steps, warmup)
+    outputs = None
+    if dump and mine:                                   # (out, status) of the last timed step, and the per-frame sizes
+        outputs = {"status": dec.status.cpu().numpy().astype(np.float64), "out_size": dec.out_size.cpu().numpy().astype(np.float64)}
+        outputs.update(sample_device_bytes(torch, dec.out, dec.out_total, "decoded_sample"))
     alg_mine = (framed.size + seg) * len(mine)
     total_alg = job.reduce(alg_mine, "sum")
     ids = [5, 10, 6]
@@ -575,7 +593,7 @@ def leg_lz4_decompress(job, args, M, total_gib, steps, warmup, seg_gib=2.0):
            "roofline": roofline(kms, alg_mine, [5, 10]) if mine else None, "clocks": clocks, "framed_by": framer,
            "total_out_bytes": seg * tiles, "tiles": tiles, "segment_bytes": seg, "segment_framed_bytes": int(framed.size), "frames_per_segment": nf,
            "tiles_per_rank": [len([t for t in range(tiles) if t % job.world == r]) for r in range(job.world)], "alg_mine": alg_mine,
-           "_keep": (src, framed)}
+           "outputs": outputs, "_keep": (src, framed)}
     del dec, dout, d_in, d_src
     torch.cuda.empty_cache()
     return res
@@ -636,7 +654,7 @@ def run_b200(args):
         cfg_par = "chunks dealt round-robin in batches of %d over %d GPU(s), no collective" % (DEAL_BATCH, job.world)
         l2 = "inputs (%.1f GiB per GPU) larger than L2" % (leg["n"] / GIB)
     else:
-        leg = leg_lz4_decompress(job, args, M, size, steps, warmup)
+        leg = leg_lz4_decompress(job, args, M, size, steps, warmup, dump=bool(args.dump_outputs))
         e2e = None if args.no_e2e else e2e_lz4_decompress(job, leg, min(e2e_steps, 5))
         cfg_par = "tiles of the framed stream dealt round-robin over %d GPU(s), no collective" % job.world
         l2 = "inputs (%.1f GiB framed per GPU) larger than L2" % (leg["alg_mine"] / GIB / 2)
@@ -681,7 +699,7 @@ def run_b200(args):
         leg.pop("_keep", None)
         del h_out
         job.torch.cuda.empty_cache()
-        xs = max(3, min(steps, 5))
+        xs = steps
         for name, gib in (("lz4-decompress", MODES["lz4-decompress"]["gib"]), ("zstd-compress", 2.0), ("zstd-mix", 2.0)):
             try:
                 Mx = MODES[name]
@@ -705,6 +723,10 @@ def run_b200(args):
                     raise                                   # a rank that skips the rest of a leg would leave the others in its collectives
                 extra[name] = {"error": repr(e)}
     line["extra"] = extra
+    if job.rank == 0 and args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in leg["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     if job.rank == 0:
         print(json.dumps(line))
     job.close()

@@ -107,14 +107,11 @@ def test_zstd_host_block_scan_on_reference_frames(level, kind):
     reference it must account for every byte of the frame, report the frame's content size and reject truncation /
     trailing bytes.  No GPU involved."""
     import _oracle as o
-    if not o.have_ref():
-        pytest.skip("oracle/_ref not built")
     import ctypes
     L = z.lib()
     n = (1 << 20) + 12345
     src = z.gen_stream(kind, n, 1 << 20)
-    rc, framed, st = o.ref_compress(o.CODEC_ZSTD, src, threads=2, level=level, chunk=1 << 19)
-    assert rc == 0
+    framed, _ = o.reference_stream(o.CODEC_ZSTD, src, level, 1 << 19)
     offs, sizes = z.scan_frames(framed)
     assert len(offs) == 3
     dsz = L.zmt_zstd_blk_desc_bytes()

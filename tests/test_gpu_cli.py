@@ -18,7 +18,7 @@ REFDIR = os.path.join(ROOT, "oracle", "_ref")
 def tool(name):
     p = os.path.join(REFDIR, name)
     if not os.path.exists(p):
-        pytest.skip(name + " not built (needs /root/reference at build time)")
+        pytest.skip(name + " not built (needs the original project's sources at build time)")
     return p
 
 

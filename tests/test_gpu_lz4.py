@@ -66,9 +66,8 @@ def test_compress_length_field_corner_cases(torch, seed, chunk):
     framed, foff = gpu_compress(torch, src, chunk)
     expect = o.orc_encode_lz4(src, chunk)
     assert framed.size == expect.size and np.array_equal(framed, expect)
-    if o.have_ref():                                  # the reference's decoder (liblz4) restores it
-        rc, back, st = o.ref_decompress(o.CODEC_LZ4, framed, src.size, threads=2)
-        assert rc == 0 and np.array_equal(back, src)
+    rc, back, _ = o.lib_decompress(o.CODEC_LZ4, framed, src.size)      # the reference's decoder (liblz4) restores it
+    assert rc == 0 and np.array_equal(back, src)
     rc, back = o.orc_decode(o.CODEC_LZ4, framed, src.size)
     assert rc == 0 and np.array_equal(back, src)
     back, status, sizes = gpu_decompress(torch, framed, chunk_sizes(src.size, chunk))
@@ -88,12 +87,10 @@ def test_compress_roundtrip_through_reference(torch, kind, chunk):
     for i in range(len(foff) - 1):
         h = framed[int(foff[i]): int(foff[i]) + 12].view("<u4")
         assert h[0] == 0x184D2A50 and h[1] == 4 and h[2] == foff[i + 1] - foff[i] - 12
-    # the reference's decoder restores the input on both of its code paths
-    if o.have_ref():
-        for T in (1, 4):
-            rc, back, st = o.ref_decompress(o.CODEC_LZ4, framed, n, threads=T)
-            assert rc == 0 and back.size == n and np.array_equal(back, src)
-            assert st[1] == len(foff) - 1            # frames
+    # the reference's decoder (liblz4, frame by frame) restores the input
+    rc, back, frames = o.lib_decompress(o.CODEC_LZ4, framed, n)
+    assert rc == 0 and back.size == n and np.array_equal(back, src)
+    assert frames == len(foff) - 1
     rc, back = o.orc_decode(o.CODEC_LZ4, framed, n)
     assert rc == 0 and np.array_equal(back, src)
 
@@ -111,20 +108,16 @@ def test_zeros_config1_container(torch):
     # LZ4F header fields equal the reference's except FLG.indep (0x6C vs 0x4C): same content size, checksum
     assert f0[12:16].tobytes().hex() == "04224d18" and f0[16] == 0x6C and f0[17] == 0x40
     assert f0[-8:].tobytes().hex() == "000000007ff93094"      # end mark + XXH32(1 MiB zeros), Appendix A
-    if o.have_ref():
-        rc, back, st = o.ref_decompress(o.CODEC_LZ4, framed, n, threads=1)
-        assert rc == 0 and back.size == n and not back.any()
+    rc, back, _ = o.lib_decompress(o.CODEC_LZ4, framed, n)
+    assert rc == 0 and back.size == n and not back.any()
 
 
 @pytest.mark.parametrize("level", [1, 3, 9])
 @pytest.mark.parametrize("kind", [z.GEN_MIX, z.GEN_TEXT, z.GEN_RANDOM, z.GEN_ZEROS])
 def test_decode_reference_streams_bit_exact(torch, level, kind):
-    if not o.have_ref():
-        pytest.skip("oracle/_ref not built")
     n, chunk = (10 << 20) + 999, 1 << 20
     src = z.gen_stream(kind, n, chunk)
-    rc, framed, st = o.ref_compress(o.CODEC_LZ4, src, threads=4, level=level, chunk=chunk)   # linked blocks, FLG 0x4C
-    assert rc == 0
+    framed, _ = o.reference_stream(o.CODEC_LZ4, src, level, chunk)   # linked blocks, FLG 0x4C
     back, status, osz = gpu_decompress(torch, framed, chunk_sizes(n, chunk))
     assert not status.any(), status
     assert back.size == n and np.array_equal(back, src)
@@ -175,26 +168,22 @@ def test_LZ4MT_compressCCtx_callbacks(torch, n, chunk):
     assert st["frames"] == nframes and st["insize"] == n and st["outsize"] == framed.size == st["out_bytes"]
     assert st["writes"] == nframes                         # exactly one fn_write per frame, in order
     assert np.array_equal(framed, o.orc_encode_lz4(src, chunk))
-    if o.have_ref():
-        rc, back, rst = o.ref_decompress(o.CODEC_LZ4, framed, n, threads=3)
-        assert rc == 0 and np.array_equal(back, src)
+    rc, back, _ = o.lib_decompress(o.CODEC_LZ4, framed, n)
+    assert rc == 0 and np.array_equal(back, src)
 
 
 @pytest.mark.parametrize("n,chunk,level", [(0, 1 << 20, 1), (1, 1 << 20, 1), ((6 << 20) + 3, 1 << 20, 1), ((70 << 20) + 1, 1 << 20, 3), (9 << 20, 4 << 20, 1)])
 def test_LZ4MT_decompressDCtx_callbacks(torch, n, chunk, level):
-    if not o.have_ref():
-        pytest.skip("oracle/_ref not built")
     src = z.gen_stream(z.GEN_MIX, n, chunk)
-    rc, framed, rst = o.ref_compress(o.CODEC_LZ4, src, threads=4, level=level, chunk=chunk)
-    assert rc == 0
+    framed, ref = o.reference_stream(o.CODEC_LZ4, src, level, chunk)
+    rst, st_r = ref["compress_stats"], ref["decompress_stats"]
     rc, back, st = z.decompress_mem(z.CODEC_LZ4, framed, n + 16, threads=4)
     assert rc == 0, z.lib().LZ4MT_getErrorString(rc)
     assert back.size == n and np.array_equal(back, src)
     # decompress statistics: Insize counts payload + 12 per frame (lz4-mt_decompress.c:238,264)
     assert st["frames"] == rst[1] and st["insize"] == framed.size and st["outsize"] == n
     # same counters as the reference's own decoder on the same stream
-    rc, back_r, st_r = o.ref_decompress(o.CODEC_LZ4, framed, n, threads=4)
-    assert rc == 0 and [st["frames"], st["insize"], st["outsize"]] == [st_r[1], st_r[2], st_r[3]]
+    assert [st["frames"], st["insize"], st["outsize"]] == [st_r[1], st_r[2], st_r[3]]
 
 
 def test_callback_error_paths(torch):

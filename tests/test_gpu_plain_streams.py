@@ -6,7 +6,9 @@ import ctypes
 import numpy as np
 import pytest
 
+import _oracle as o
 import zstdmt_b200 as z
+from _oracle import LZ4FPrefs
 
 pytestmark = pytest.mark.gpu
 
@@ -16,12 +18,6 @@ def gpu():
     import torch
     if not torch.cuda.is_available():
         pytest.skip("no CUDA device")
-
-
-class LZ4FPrefs(ctypes.Structure):
-    _fields_ = [("blockSizeID", ctypes.c_int), ("blockMode", ctypes.c_int), ("contentChecksumFlag", ctypes.c_int), ("frameType", ctypes.c_int),
-                ("contentSize", ctypes.c_ulonglong), ("dictID", ctypes.c_uint), ("blockChecksumFlag", ctypes.c_int),
-                ("compressionLevel", ctypes.c_int), ("autoFlush", ctypes.c_uint), ("favorDecSpeed", ctypes.c_uint), ("reserved", ctypes.c_uint * 3)]
 
 
 def lz4f(data, **kw):
@@ -180,23 +176,26 @@ def test_plain_zstd_streamed_frames_without_content_size(gpu, checksum):
     assert np.array_equal(back, np.concatenate([a, b]))
 
 
+def zstdmt_style_stream(src, chunk):
+    """A 9-byte empty zstd frame, then [12-byte skippable header][zstd frame of one chunk]*."""
+    parts = [np.frombuffer(bytes.fromhex("28b52ffd2000010000"), np.uint8)]
+    for a in range(0, src.size, chunk):
+        f = zstd1(src[a:a + chunk], 3)
+        parts += [np.frombuffer((0x184D2A50).to_bytes(4, "little") + (4).to_bytes(4, "little") + int(f.size).to_bytes(4, "little"), np.uint8), f]
+    return np.concatenate(parts)
+
+
 def test_zstdmt_style_stream(gpu):
     """zstdmt-style framing: a 9-byte empty zstd frame, then [12-byte skippable header][zstd frame]* — the second branch of
     the stream sniffing (zstd-mt_decompress.c:745-749, first-frame fix-up :231-263)."""
     n, chunk = (3 << 20) + 77, 1 << 20
     src = z.gen_stream(z.GEN_MIX, n, chunk)
-    frames = [zstd1(src[o:o + chunk], 3) for o in range(0, n, chunk)]
-    parts = [np.frombuffer(bytes.fromhex("28b52ffd2000010000"), np.uint8)]
-    for f in frames:
-        parts += [np.frombuffer((0x184D2A50).to_bytes(4, "little") + (4).to_bytes(4, "little") + int(f.size).to_bytes(4, "little"), np.uint8), f]
-    stream = np.concatenate(parts)
+    stream = zstdmt_style_stream(src, chunk)
     rc, back, st = z.decompress_mem(z.CODEC_ZSTD, stream, n + 16, threads=4)
     assert rc == 0, z.lib().ZSTDCB_getErrorString(rc)
-    assert np.array_equal(back, src) and st["frames"] == len(frames)
-    import _oracle as o
-    if o.have_ref():                                                    # the reference accepts the very same bytes
-        rc, back_r, _ = o.ref_decompress(o.CODEC_ZSTD, stream, n, threads=4)
-        assert rc == 0 and np.array_equal(back_r, src)
+    assert np.array_equal(back, src) and st["frames"] == -(-n // chunk)
+    ref = o.reference_decoded(o.CODEC_ZSTD, stream)                     # the reference accepted the very same bytes
+    assert ref["rc"] == 0 and ref["out_bytes"] == n and ref["sha256"] == o.sha256(src)
 
 
 @pytest.mark.parametrize("codec", ["lz4", "zstd"])

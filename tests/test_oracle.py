@@ -1,6 +1,7 @@
 """CPU tests: pin the oracle (oracle/*.c) against the golden vectors of SURVEY.md Appendix A
-(captured from the real reference build) and, when oracle/_ref is present, against the real
-reference itself (liblz4 1.9.4 / libzstd 1.5.5 behind the unmodified lib/*-mt_*.c)."""
+(captured from the real reference build) and against streams of the real reference itself
+(liblz4 1.9.4 / libzstd 1.5.5 behind the unmodified lib/*-mt_*.c), re-made through the same
+library calls and checked against digests of the reference's output (tests/golden/reference_streams.json)."""
 import os
 
 import numpy as np
@@ -10,7 +11,6 @@ import _oracle as o
 import zstdmt_b200 as z
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-needs_ref = pytest.mark.skipif(not o.have_ref(), reason="oracle/_ref not built")
 
 
 def hexb(s):
@@ -67,36 +67,31 @@ def test_golden_fixture_files():
         assert o.xxh32(framed) == case["xxh32_framed"], case
 
 
-@needs_ref
 def test_ref_lz4_zeros_1mib_matches_appendix_a():
-    rc, f, st = o.ref_compress(o.CODEC_LZ4, np.zeros(1 << 20, np.uint8), threads=1, level=1)
-    assert rc == 0 and f.size == 4356
+    f, _ = o.reference_stream(o.CODEC_LZ4, np.zeros(1 << 20, np.uint8), 1, 1 << 20)
+    assert f.size == 4356
     assert f[:28].tobytes().hex() == "502a4d1804000000f810000004224d184c400000100000000000880b010000"[:56]
     assert f[-8:].tobytes().hex() == "000000007ff93094"
     rc, out = o.orc_decode(o.CODEC_LZ4, f, 1 << 20)
     assert rc == 0 and out.size == 1 << 20 and not out.any()
 
 
-@needs_ref
 @pytest.mark.parametrize("codec,level", [(1, 1), (1, 3), (2, 1), (2, 3), (2, 9)])
 @pytest.mark.parametrize("kind", [z.GEN_MIX, z.GEN_TEXT, z.GEN_RANDOM, z.GEN_ZEROS])
 def test_oracle_decodes_reference_streams(codec, level, kind):
     n = (5 << 20) + 12345 if kind == z.GEN_MIX else (1 << 20) + 77
     src = z.gen_stream(kind, n, 1 << 20)
-    rc, f, st = o.ref_compress(codec, src, threads=2, level=level)
-    assert rc == 0
+    f, _ = o.reference_stream(codec, src, level, 1 << 20)
     rc, out = o.orc_decode(codec, f, n)
     assert rc == 0 and out.size == n and np.array_equal(out, src)
 
 
-@needs_ref
 @pytest.mark.parametrize("n", [0, 1, 11, 12, 13, 39, 40, 65535, 65536, 65537, (1 << 20) - 1, (1 << 20) + 1])
 def test_b200_encoder_twin_roundtrips_through_reference(n):
     src = z.gen_stream(z.GEN_MIX, n, 1 << 20, first=1)
     f = o.orc_encode_lz4(src)
-    for T in (1, 3):
-        rc, out, st = o.ref_decompress(o.CODEC_LZ4, f, n, threads=T)
-        assert rc == 0 and out.size == n and np.array_equal(out, src)
+    rc, out, frames = o.lib_decompress(o.CODEC_LZ4, f, n)           # liblz4, the reference's decoder
+    assert rc == 0 and out.size == n and np.array_equal(out, src) and frames == max(1, -(-n // (1 << 20)))
     rc, out = o.orc_decode(o.CODEC_LZ4, f, n)
     assert rc == 0 and np.array_equal(out, src)
 
@@ -122,6 +117,5 @@ def test_b200_encoder_twin_length_field_corner_cases(chunk):
     framed = o.orc_encode_lz4(src, chunk)
     rc, back = o.orc_decode(o.CODEC_LZ4, framed, src.size)
     assert rc == 0 and np.array_equal(back, src)
-    if o.have_ref():
-        rc, back, st = o.ref_decompress(o.CODEC_LZ4, framed, src.size, threads=2)
-        assert rc == 0 and np.array_equal(back, src)
+    rc, back, _ = o.lib_decompress(o.CODEC_LZ4, framed, src.size)
+    assert rc == 0 and np.array_equal(back, src)
