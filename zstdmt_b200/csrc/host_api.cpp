@@ -32,21 +32,6 @@
 #include <vector>
 #include "zmt_dev.h"
 
-extern "C" {
-size_t   zmt_zstdc_workspace_bytes(uint32_t nchunks, uint32_t chunk_size);
-uint64_t zmt_zstdc_out_bound(uint32_t nchunks, uint32_t chunk_size);
-int      zmt_zstd_compress_device(const void*, uint64_t, uint32_t, const uint32_t*, uint32_t, void*, void*, uint64_t*, void*);
-size_t   zmt_zstd_blk_desc_bytes(void);
-int      zmt_zstd_scan_frame_host(const uint8_t* frame, size_t n, uint64_t base_off, uint32_t frame_idx, void* blocks_out, uint32_t* nblocks_io,
-                                  uint32_t max_blocks, uint64_t* scratch_used, uint64_t* content_size, uint32_t* needs_seq);
-int      zmt_zstd_scan_frame_host2(const uint8_t* frame, size_t n, uint64_t base_off, uint32_t frame_idx, void* blocks_out, uint32_t* nblocks_io,
-                                   uint32_t max_blocks, uint64_t* scratch_used, uint64_t* content_size, uint32_t* needs_seq, size_t* consumed);
-size_t   zmt_zstdd_workspace_bytes(uint32_t nframes, uint32_t nblocks, uint64_t scratch_bytes);
-int      zmt_zstd_decompress_device(const void* d_in, const void* d_blocks, uint32_t nblocks, const uint32_t* d_frame_first_blk, const uint64_t* d_expect,
-                                    const uint32_t* d_frame_seq, uint32_t nframes, void* d_out, const uint64_t* d_out_off, uint64_t* d_out_size, uint32_t* d_status,
-                                    void* d_work, void* stream);
-}
-
 namespace {
 
 // ------------------------------------------------------------------ generic boundary types
@@ -185,11 +170,18 @@ struct DeviceRestore {
 };
 
 // ------------------------------------------------------------------ optional stage timing (ZSTDMT_B200_TRACE=1)
-struct StageClock {
-    double cb = 0, wait = 0, gpu = 0;       // seconds: inside callbacks / waiting for a slot or queue / CUDA sync + copies
-    static double now() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
-};
 inline bool trace_on() { static int on = -1; if (on < 0) on = getenv("ZSTDMT_B200_TRACE") ? 1 : 0; return on == 1; }
+inline double now() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
+
+// seconds per stage of one call: inside callbacks / waiting for a slot / the zstd host block scan / waiting for the device
+struct Clocks { double rd_total = 0, rd_cb = 0, rd_scan = 0, rd_wait = 0, sub_enqueue = 0, sub_wait = 0, wr_gpu = 0, wr_cb = 0, wr_wait = 0; };
+
+// adds its own lifetime to `acc`; the clock is only read under ZSTDMT_B200_TRACE=1
+struct Timed {
+    double* acc; double t0;
+    explicit Timed(double& a) : acc(trace_on() ? &a : nullptr), t0(acc ? now() : 0) {}
+    ~Timed() { if (acc) *acc += now() - t0; }
+};
 
 // ------------------------------------------------------------------ device codec table
 struct CodecOps {
@@ -198,7 +190,6 @@ struct CodecOps {
     int      (*compress)(const void*, uint64_t, uint32_t, const uint32_t*, uint32_t, void*, void*, uint64_t*, void*);
 };
 
-
 const CodecOps* codec_ops(int codec)
 {
     static const CodecOps lz4 = { zmt_lz4c_workspace_bytes, zmt_lz4c_out_bound, zmt_lz4_compress_device };
@@ -206,78 +197,62 @@ const CodecOps* codec_ops(int codec)
     return codec == CODEC_LZ4 ? &lz4 : &zstd;
 }
 
+// ------------------------------------------------------------------ batch tables
+// One entry per chunk (compress) or frame (decompress); every field means the same in both directions and codecs.
+// Layout (cap entries): u64 frame_off, out_off, out_size, expect [cap+1] | u32 frame_len, frame_flags, status [cap] | u32 first_blk [cap+1]
+struct Tables {
+    uint64_t *frame_off, *out_off;    // the frame's 12-byte header in the slot's input (decompress) / its output; out_off[n] = total
+    uint64_t *out_size, *expect;      // bytes the device decoded / zstd: header content size, ~0 when that is only a bound
+    uint32_t *frame_len, *frame_flags;// input bytes (chunk / frame payload) / zstd: scan flags (sequential pass, checksum, no size)
+    uint32_t *status, *first_blk;     // ZMT_ST_* of the frame / zstd: its first block descriptor; first_blk[n] = total
+};
+inline size_t tables_bytes(size_t cap) { return 4 * (cap + 1) * 8 + 3 * cap * 4 + (cap + 1) * 4 + 64; }
+inline Tables tables_at(uint8_t* base, size_t cap)
+{
+    Tables t;
+    t.frame_off = (uint64_t*)base; t.out_off = t.frame_off + cap + 1; t.out_size = t.out_off + cap + 1; t.expect = t.out_size + cap + 1;
+    t.frame_len = (uint32_t*)(t.expect + cap + 1); t.frame_flags = t.frame_len + cap; t.status = t.frame_flags + cap; t.first_blk = t.status + cap;
+    return t;
+}
+
+// lz4 decode block table: every frame owns max(1, ceil(out / 64 KiB)) slots
+inline uint32_t lz4_block_slots(uint64_t out_bytes) { const uint64_t nb = (out_bytes + 65535) / 65536; return nb ? (uint32_t)nb : 1; }
+inline uint32_t lz4_slot_cap(size_t out_cap, size_t tab_cap) { return (uint32_t)(out_cap / 65536 + tab_cap + 1); }
+
 // ------------------------------------------------------------------ staging slots
+struct SlotCaps {
+    size_t in = 0, out = 0, work = 0, tab = 0;   // bytes of input, output and workspace; entries of the batch tables
+    uint32_t blk = 0;                            // zstd decompress: block descriptors
+    uint64_t scr = 0;                            // zstd decompress: entropy scratch bytes the workspace was sized for
+};
+
 struct Slot {
     int dev = 0;
     cudaStream_t stream = nullptr;
     cudaEvent_t ev = nullptr, evp[2] = { nullptr, nullptr };       // evp: decompress writer, output pieces in flight
     uint8_t *h_in = nullptr, *h_out = nullptr, *d_in = nullptr, *d_out = nullptr, *d_work = nullptr;
-    size_t in_cap = 0, out_cap = 0, work_cap = 0, tab_cap = 0;   // tab_cap: entries in the tables below
-    // tables: pinned host mirror + device copy, one allocation each
-    uint8_t *h_tab = nullptr, *d_tab = nullptr; size_t tab_bytes = 0;
+    uint8_t *h_tab = nullptr, *d_tab = nullptr; size_t tab_bytes = 0;      // batch tables: pinned host mirror + device copy
+    uint8_t *h_blk = nullptr, *d_blk = nullptr;                             // zstd block descriptors built by the reader
+    SlotCaps cap;
+    bool ok = false;
+    bool host_alias = false;     // h_in / h_out are borrowed from another slot of the same context (never freed here)
     // batch contents
     uint32_t n = 0;              // chunks / frames in this batch
-    uint32_t nslots = 1;         // lz4 decompress: block-table slots of this batch (sum over frames of max(1, ceil(out / 64 KiB)))
-    uint64_t scr_cap = 0;        // zstd decompress: entropy scratch bytes the workspace was sized for
-    // zstd decompress: block descriptors built by the reader (pinned) + device copy, scratch demand of the batch
-    uint8_t *h_blk = nullptr, *d_blk = nullptr; uint32_t blk_cap = 0, nblk = 0; uint64_t scratch_used = 0;
+    uint32_t nslots = 1;         // lz4 decompress: block-table slots of this batch (sum of lz4_block_slots over frames)
+    uint32_t nblk = 0;           // zstd decompress: block descriptors of this batch
     size_t in_used = 0, out_used = 0;
     int state = 0;               // 0 free, 1 filled, 2 submitted
-    bool ok = false;
-    bool host_alias = false;     // h_in / h_out are borrowed from another slot of the same context (never pooled, never freed here)
 };
-
-// table layout (entries = tab_cap):  u64 a[cap+1] | u64 b[cap+1] | u64 c[cap+1] | u64 f[cap+1] | u32 d[cap] | u32 e[cap] | u32 g[cap+1]
-struct Tables { uint64_t *a, *b, *c, *f; uint32_t *d, *e, *g; };
-inline size_t tables_bytes(size_t cap) { return 4 * (cap + 1) * 8 + 2 * cap * 4 + (cap + 1) * 4 + 64; }
-inline Tables tables_at(uint8_t* base, size_t cap)
-{
-    Tables t; t.a = (uint64_t*)base; t.b = t.a + cap + 1; t.c = t.b + cap + 1; t.f = t.c + cap + 1;
-    t.d = (uint32_t*)(t.f + cap + 1); t.e = t.d + cap; t.g = t.e + cap; return t;
-}
-
-// lz4 decode block table capacity of a slot: every frame owns max(1, ceil(out / 64 KiB)) slots
-inline uint32_t lz4_slot_cap(size_t out_cap, size_t tab_cap) { return (uint32_t)(out_cap / 65536 + tab_cap + 1); }
 
 void slot_free_raw(Slot& s)
 {
     cudaSetDevice(s.dev);
     if (s.stream) cudaStreamSynchronize(s.stream);
-    if (s.h_in) cudaFreeHost(s.h_in);
-    if (s.h_out) cudaFreeHost(s.h_out);
-    if (s.h_tab) cudaFreeHost(s.h_tab);
-    if (s.d_in) cudaFree(s.d_in);
-    if (s.d_out) cudaFree(s.d_out);
-    if (s.d_work) cudaFree(s.d_work);
-    if (s.d_tab) cudaFree(s.d_tab);
-    if (s.h_blk) cudaFreeHost(s.h_blk);
-    if (s.d_blk) cudaFree(s.d_blk);
-    if (s.ev) cudaEventDestroy(s.ev);
-    for (int k = 0; k < 2; k++) if (s.evp[k]) cudaEventDestroy(s.evp[k]);
+    for (uint8_t* p : { s.h_in, s.h_out, s.h_tab, s.h_blk }) if (p) cudaFreeHost(p);
+    for (uint8_t* p : { s.d_in, s.d_out, s.d_work, s.d_tab, s.d_blk }) if (p) cudaFree(p);
+    for (cudaEvent_t e : { s.ev, s.evp[0], s.evp[1] }) if (e) cudaEventDestroy(e);
     if (s.stream) cudaStreamDestroy(s.stream);
     s = Slot();
-}
-
-bool slot_alloc_raw(Slot& s, int dev, size_t in_cap, size_t out_cap, size_t work_cap, size_t tab_cap)
-{
-    s.dev = dev;
-    if (cudaSetDevice(dev) != cudaSuccess) return false;
-    const ScopedAffinity bind(device_local_cpus(dev));     // first touch of the pinned rings happens on the GPU's node
-    bool ok = true;
-    ok = ok && cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking) == cudaSuccess;
-    ok = ok && cudaEventCreateWithFlags(&s.ev, cudaEventDisableTiming) == cudaSuccess;
-    for (int k = 0; k < 2; k++) ok = ok && cudaEventCreateWithFlags(&s.evp[k], cudaEventDisableTiming) == cudaSuccess;
-    ok = ok && cudaHostAlloc((void**)&s.h_in, in_cap + 64, cudaHostAllocPortable) == cudaSuccess;
-    ok = ok && cudaHostAlloc((void**)&s.h_out, out_cap + 64, cudaHostAllocPortable) == cudaSuccess;
-    ok = ok && cudaMalloc((void**)&s.d_in, in_cap + 256) == cudaSuccess;
-    ok = ok && cudaMalloc((void**)&s.d_out, out_cap + 256) == cudaSuccess;
-    ok = ok && cudaMalloc((void**)&s.d_work, work_cap + 256) == cudaSuccess;
-    s.tab_bytes = tables_bytes(tab_cap);
-    ok = ok && cudaHostAlloc((void**)&s.h_tab, s.tab_bytes, cudaHostAllocPortable) == cudaSuccess;
-    ok = ok && cudaMalloc((void**)&s.d_tab, s.tab_bytes) == cudaSuccess;
-    s.in_cap = in_cap; s.out_cap = out_cap; s.work_cap = work_cap; s.tab_cap = tab_cap; s.ok = ok;
-    if (!ok) { cudaGetLastError(); slot_free_raw(s); }
-    return ok;
 }
 
 // Process-wide pool of staging slots: pinned allocations cost ~0.1 s per context otherwise (the reference's
@@ -287,69 +262,59 @@ std::mutex g_pool_mu;
 std::vector<Slot> g_pool;
 const size_t kPoolMax = 16;
 
-bool slot_alloc(Slot& s, int dev, size_t in_cap, size_t out_cap, size_t work_cap, size_t tab_cap)
+// Takes a slot of at least `want` (the same table capacity) on `dev` from the pool, or allocates one.  With a
+// `host_owner` the slot borrows that slot's pinned staging buffers and has only its device side (a call over more
+// devices than it keeps batches in flight: the host ring stays 4 x 8 MiB — cache-resident for the callbacks' memcpy —
+// while every device has its own device-side buffers).
+bool slot_acquire(Slot& s, int dev, const SlotCaps& want, const Slot* host_owner)
 {
+    const bool own_host = host_owner == nullptr;
+    bool found = false;
     {
         std::lock_guard<std::mutex> g(g_pool_mu);
-        for (size_t i = 0; i < g_pool.size(); i++) {
-            Slot& c = g_pool[i];
-            if (c.h_in && c.dev == dev && c.in_cap >= in_cap && c.out_cap >= out_cap && c.work_cap >= work_cap && c.tab_cap == tab_cap) {
-                s = c; g_pool.erase(g_pool.begin() + (long)i);
-                s.state = 0; s.n = 0; s.in_used = s.out_used = 0;
-                return true;
+        for (size_t i = 0; i < g_pool.size() && !found; i++) {
+            const Slot& c = g_pool[i];
+            if (c.dev == dev && (c.h_in != nullptr) == own_host && c.cap.in >= want.in && c.cap.out >= want.out && c.cap.work >= want.work &&
+                c.cap.blk >= want.blk && c.cap.tab == want.tab) {
+                s = c; g_pool.erase(g_pool.begin() + (long)i); found = true;
             }
         }
     }
-    return slot_alloc_raw(s, dev, in_cap, out_cap, work_cap, tab_cap);
-}
-
-// A slot whose pinned staging buffers are those of `owner` (a call over more devices than it keeps batches in flight: the
-// host ring stays 4 x 8 MiB — cache-resident for the callbacks' memcpy — while every device has its own device-side buffers).
-bool slot_alloc_alias(Slot& s, const Slot& owner, int dev, size_t in_cap, size_t out_cap, size_t work_cap, size_t tab_cap)
-{
-    {
-        std::lock_guard<std::mutex> g(g_pool_mu);                       // a pooled device-only slot of a previous call
-        for (size_t i = 0; i < g_pool.size(); i++) {
-            Slot& c = g_pool[i];
-            if (!c.h_in && c.dev == dev && c.in_cap >= in_cap && c.out_cap >= out_cap && c.work_cap >= work_cap && c.tab_cap == tab_cap) {
-                s = c; g_pool.erase(g_pool.begin() + (long)i);
-                s.state = 0; s.n = 0; s.in_used = s.out_used = 0;
-                s.h_in = owner.h_in; s.h_out = owner.h_out; s.host_alias = true;
-                return true;
-            }
+    if (!found) {
+        s = Slot(); s.dev = dev;
+        if (cudaSetDevice(dev) != cudaSuccess) return false;
+        const ScopedAffinity bind(own_host ? device_local_cpus(dev) : CpuSet());     // first touch of the pinned rings happens on the GPU's node
+        const size_t blk_bytes = (size_t)want.blk * zmt_zstd_blk_desc_bytes();
+        s.tab_bytes = tables_bytes(want.tab);
+        bool ok = cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking) == cudaSuccess;
+        ok = ok && cudaEventCreateWithFlags(&s.ev, cudaEventDisableTiming) == cudaSuccess;
+        for (int k = 0; k < 2; k++) ok = ok && cudaEventCreateWithFlags(&s.evp[k], cudaEventDisableTiming) == cudaSuccess;
+        if (own_host) {
+            ok = ok && cudaHostAlloc((void**)&s.h_in, want.in + 64, cudaHostAllocPortable) == cudaSuccess;
+            ok = ok && cudaHostAlloc((void**)&s.h_out, want.out + 64, cudaHostAllocPortable) == cudaSuccess;
         }
+        ok = ok && cudaMalloc((void**)&s.d_in, want.in + 256) == cudaSuccess;
+        ok = ok && cudaMalloc((void**)&s.d_out, want.out + 256) == cudaSuccess;
+        ok = ok && cudaMalloc((void**)&s.d_work, want.work + 256) == cudaSuccess;
+        ok = ok && cudaHostAlloc((void**)&s.h_tab, s.tab_bytes, cudaHostAllocPortable) == cudaSuccess;
+        ok = ok && cudaMalloc((void**)&s.d_tab, s.tab_bytes) == cudaSuccess;
+        if (want.blk) {
+            ok = ok && cudaHostAlloc((void**)&s.h_blk, blk_bytes, cudaHostAllocPortable) == cudaSuccess;
+            ok = ok && cudaMalloc((void**)&s.d_blk, blk_bytes) == cudaSuccess;
+        }
+        s.cap = want; s.ok = ok;
+        if (!ok) { cudaGetLastError(); slot_free_raw(s); return false; }
     }
-    s.dev = dev;
-    if (cudaSetDevice(dev) != cudaSuccess) return false;
-    bool ok = true;
-    ok = ok && cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking) == cudaSuccess;
-    ok = ok && cudaEventCreateWithFlags(&s.ev, cudaEventDisableTiming) == cudaSuccess;
-    for (int k = 0; k < 2; k++) ok = ok && cudaEventCreateWithFlags(&s.evp[k], cudaEventDisableTiming) == cudaSuccess;
-    ok = ok && cudaMalloc((void**)&s.d_in, in_cap + 256) == cudaSuccess;
-    ok = ok && cudaMalloc((void**)&s.d_out, out_cap + 256) == cudaSuccess;
-    ok = ok && cudaMalloc((void**)&s.d_work, work_cap + 256) == cudaSuccess;
-    s.tab_bytes = tables_bytes(tab_cap);
-    ok = ok && cudaHostAlloc((void**)&s.h_tab, s.tab_bytes, cudaHostAllocPortable) == cudaSuccess;
-    ok = ok && cudaMalloc((void**)&s.d_tab, s.tab_bytes) == cudaSuccess;
-    s.in_cap = in_cap; s.out_cap = out_cap; s.work_cap = work_cap; s.tab_cap = tab_cap; s.ok = ok;
-    if (!ok) { cudaGetLastError(); slot_free_raw(s); return false; }
-    s.h_in = owner.h_in; s.h_out = owner.h_out; s.host_alias = true;
+    s.cap.scr = want.scr;              // what the caller sized the workspace for
+    s.state = 0; s.n = 0; s.in_used = s.out_used = 0;
+    if (!own_host) { s.h_in = host_owner->h_in; s.h_out = host_owner->h_out; s.host_alias = true; }
     return true;
 }
 
-void slot_free(Slot& s)
+// Back to the pool (a borrower without the owner's buffers, as a device-only slot), or freed.
+void slot_release(Slot& s)
 {
-    if (s.host_alias) {
-        // hand the borrowed buffers back (they belong to the owner slot); the device side goes to the pool as a device-only slot
-        s.h_in = nullptr; s.h_out = nullptr; s.host_alias = false;
-        if (s.ok) {
-            cudaSetDevice(s.dev);
-            if (s.stream) cudaStreamSynchronize(s.stream);
-            std::lock_guard<std::mutex> g(g_pool_mu);
-            if (g_pool.size() < kPoolMax && !getenv("ZSTDMT_B200_NO_POOL")) { g_pool.push_back(s); s = Slot(); return; }
-        }
-        slot_free_raw(s); return;
-    }
+    if (s.host_alias) { s.h_in = nullptr; s.h_out = nullptr; s.host_alias = false; }
     if (s.ok) {
         cudaSetDevice(s.dev);
         if (s.stream) cudaStreamSynchronize(s.stream);
@@ -357,20 +322,6 @@ void slot_free(Slot& s)
         if (g_pool.size() < kPoolMax && !getenv("ZSTDMT_B200_NO_POOL")) { g_pool.push_back(s); s = Slot(); return; }
     }
     slot_free_raw(s);
-}
-
-bool slot_ensure_blocks(Slot& s, uint32_t cap)
-{
-    if (s.blk_cap >= cap) return true;
-    cudaSetDevice(s.dev);
-    if (s.h_blk) cudaFreeHost(s.h_blk);
-    if (s.d_blk) cudaFree(s.d_blk);
-    s.h_blk = s.d_blk = nullptr; s.blk_cap = 0;
-    const size_t bytes = (size_t)cap * zmt_zstd_blk_desc_bytes();
-    if (cudaHostAlloc((void**)&s.h_blk, bytes, cudaHostAllocPortable) != cudaSuccess) { cudaGetLastError(); return false; }
-    if (cudaMalloc((void**)&s.d_blk, bytes) != cudaSuccess) { cudaGetLastError(); return false; }
-    s.blk_cap = cap;
-    return true;
 }
 
 // ------------------------------------------------------------------ pipeline state shared by the 3 threads
@@ -381,6 +332,7 @@ struct Pipe {
     size_t fill_seq = 0, submit_seq = 0, write_seq = 0;
     bool reader_done = false;
     size_t error = 0;                 // first error wins
+    Clocks clk;
     void fail(size_t e) { std::lock_guard<std::mutex> g(mu); if (!error) error = e; cv.notify_all(); }
 };
 
@@ -397,9 +349,132 @@ struct Ctx {
 
 void ctx_release_slots(Ctx* c)
 {
-    for (auto& s : c->pipe.slots) if (s.ok && s.host_alias) slot_free(s);         // borrowers before the owners of the host buffers
-    for (auto& s : c->pipe.slots) if (s.ok) slot_free(s);
+    for (auto& s : c->pipe.slots) if (s.ok && s.host_alias) slot_release(s);      // borrowers before the owners of the host buffers
+    for (auto& s : c->pipe.slots) if (s.ok) slot_release(s);
     c->pipe.slots.clear();
+}
+
+// the devices of a context, chosen on its first call (ZSTDMT_GPUS)
+bool ctx_devices(Ctx* c)
+{
+    if (c->pipe.slots.empty()) c->devs = env_devices();
+    if (c->devs.empty()) { c->lib_errcode = ZMT_ST_CUDA; return false; }
+    return true;
+}
+
+// pinned staging slots (batches in flight) of a call: one per host thread asked for, 2..4
+size_t host_slots(const Ctx* c) { return c->threads >= 4 ? 4 : c->threads >= 3 ? 3 : 2; }
+
+// a frame status as the call's error: a frame cut short is "could not decompress frame", anything else the library's
+size_t status_error(Ctx* c, uint32_t st)
+{
+    c->lib_errcode = st;
+    return (st == ZMT_ST_TRUNCATED || st == ZMT_ST_TRAILING) ? c->E->frame_decompress : c->E->library;
+}
+
+// reads exactly `want` bytes unless EOF; returns 0 ok / error; *got = delivered
+size_t read_some(Ctx* c, GenRdWr* rw, void* dst, size_t want, size_t* got)
+{
+    GenBuffer b; b.buf = dst; b.size = want; b.allocated = want;
+    int rv;
+    { const Timed t(c->pipe.clk.rd_cb); rv = rw->fn_read(rw->arg_read, &b); }
+    if (rv != 0) return mt_error(*c->E, rv);
+    if (b.size > want) return c->E->read_fail;
+    *got = b.size; return 0;
+}
+
+size_t write_all(Ctx* c, GenRdWr* rw, void* src, size_t n)
+{
+    GenBuffer b; b.buf = src; b.size = n; b.allocated = n;
+    int rv;
+    { const Timed t(c->pipe.clk.wr_cb); rv = rw->fn_write(rw->arg_write, &b); }
+    if (rv != 0) return mt_error(*c->E, rv);
+    c->outsize += b.size;
+    return 0;
+}
+
+// ------------------------------------------------------------------ the pipeline
+// One call over c->pipe.slots, batch q in slot q % N:
+//   fill(slot, last)  reader thread, every fn_read call; puts slot.n > 0 items into the slot, or 0 at the end of the
+//                     input; sets `last` when the input ended behind this batch
+//   submit(slot)      calling thread: H2D, kernels, D2H of the tables, event slot.ev recorded
+//   drain(slot)       writer thread, after slot.ev: every fn_write call, strictly in order
+// Each returns 0 or the call's error; the first error stops all three.  Batch q + in_flight is not filled before batch
+// q is written (slots that share their host buffers).  Reads never overlap reads, writes never overlap writes.
+template <class Fill, class Submit, class Drain>
+size_t run_pipeline(Ctx* c, size_t in_flight, Fill fill, Submit submit, Drain drain)
+{
+    Pipe& P = c->pipe;
+    const size_t N = P.slots.size();
+    const double slot_mib = (double)P.slots[0].cap.in / (1 << 20);
+    P.fill_seq = P.submit_seq = P.write_seq = 0; P.reader_done = false; P.error = 0; P.clk = Clocks();
+    for (auto& s : P.slots) s.state = 0;
+
+    // the slot of sequence number `seq` once it is in `state`; nullptr on an error or when the reader has ended before it
+    auto await = [&](const size_t& seq, int state, double& clk) -> Slot* {
+        const Timed t(clk);
+        std::unique_lock<std::mutex> lk(P.mu);
+        Slot* s = &P.slots[seq % N];
+        P.cv.wait(lk, [&] {
+            if (P.error) return true;
+            if (state == 0) return s->state == 0 && P.fill_seq - P.write_seq < in_flight;
+            return s->state == state || (P.reader_done && seq == P.fill_seq);
+        });
+        return (P.error || s->state != state) ? nullptr : s;
+    };
+    auto advance = [&](Slot* s, int state, size_t& seq) {
+        { std::lock_guard<std::mutex> g(P.mu); s->state = state; seq++; }
+        P.cv.notify_all();
+    };
+
+    const CpuSet host_cpus = common_local_cpus(c->devs);
+    std::thread reader([&]() {
+        const ScopedAffinity bind(host_cpus);
+        {
+            const Timed t(P.clk.rd_total);
+            for (bool last = false; !last;) {
+                Slot* s = await(P.fill_seq, 0, P.clk.rd_wait);
+                if (!s) break;
+                const size_t e = fill(*s, last);
+                if (e) { P.fail(e); break; }
+                if (s->n == 0) break;
+                advance(s, 1, P.fill_seq);
+            }
+        }
+        { std::lock_guard<std::mutex> g(P.mu); P.reader_done = true; }
+        P.cv.notify_all();
+    });
+    std::thread writer([&]() {
+        const ScopedAffinity bind(host_cpus);
+        for (;;) {
+            Slot* s = await(P.write_seq, 2, P.clk.wr_wait);
+            if (!s) break;
+            cudaSetDevice(s->dev);
+            cudaError_t ce;
+            { const Timed t(P.clk.wr_gpu); ce = cudaEventSynchronize(s->ev); }
+            const size_t e = ce == cudaSuccess ? drain(*s) : (c->lib_errcode = ZMT_ST_CUDA, c->E->library);
+            if (e) { P.fail(e); break; }
+            advance(s, 0, P.write_seq);
+        }
+    });
+    for (;;) {
+        Slot* s = await(P.submit_seq, 1, P.clk.sub_wait);
+        if (!s) break;
+        size_t e;
+        { const Timed t(P.clk.sub_enqueue); cudaSetDevice(s->dev); e = submit(*s); }
+        if (s->dev >= 0 && s->dev < 64) g_dev_batches[s->dev]++;
+        if (e) { P.fail(e); break; }
+        advance(s, 2, P.submit_seq);
+    }
+    reader.join(); writer.join();
+    for (auto& s : P.slots) if (s.ok) { cudaSetDevice(s.dev); cudaStreamSynchronize(s.stream); }
+    if (trace_on()) {
+        const Clocks& k = P.clk;
+        fprintf(stderr, "[zstdmt_b200] %s: reader total %.3fs cb %.3fs scan %.3fs wait %.3fs | submit enqueue %.3fs wait %.3fs | "
+                        "writer gpu-wait %.3fs cb %.3fs wait %.3fs | slots %zu x %.1f MiB\n", c->is_comp ? "compress" : "decompress",
+                k.rd_total, k.rd_cb, k.rd_scan, k.rd_wait, k.sub_enqueue, k.sub_wait, k.wr_gpu, k.wr_cb, k.wr_wait, N, slot_mib);
+    }
+    return P.error;
 }
 
 // ------------------------------------------------------------------ compression
@@ -408,167 +483,118 @@ size_t compress_run(Ctx* c, GenRdWr* rw)
     const DeviceRestore restore_device;
     const ErrCodes& E = *c->E;
     const CodecOps* ops = codec_ops(c->codec);
-    if (!ops->compress || !ops->c_work || !ops->c_bound) { c->lib_errcode = ZMT_ST_UNSUPPORTED; return E.library; }
     Pipe& P = c->pipe;
     const size_t chunk = c->inputsize;
     // Slots in flight: the call is bound by the serialised callbacks (one memcpy stream); a GPU turns a batch around in a
-    // fraction of the time the reader needs to fill the next one, so more devices do not need more slots per device — one each
-    // is enough.  Measured on the 2-socket Xeon hosts of the B200 pool (one GPU, 4 GiB, GB/s end to end): 4 slots x 8 MiB 18.2
+    // fraction of the time the reader needs to fill the next one, so more devices do not need more batches in flight.
+    // Measured on the 2-socket Xeon hosts of the B200 pool (one GPU, 4 GiB, GB/s end to end): 4 slots x 8 MiB 18.2
     // (the default), 4 x 4 MiB 15.8, 4 x 16 MiB 14.4, 8 x 8 MiB 13.7, 8 x 4 MiB 9.9, 16 x 2 MiB 5.2: a ring that outgrows the
-    // last-level cache slows the callbacks' memcpy, and small batches pay the per-batch launch + copy latency.  A call over 8
-    // devices therefore runs 8 x 8 MiB (14.3 GB/s): sharing a 4-slot host ring between 8 device-side slots is the open lead.
-    if (P.slots.empty()) {
-        c->devs = env_devices();
-        if (c->devs.empty()) { c->lib_errcode = ZMT_ST_CUDA; return E.library; }
-    }
-    const size_t base_slots = c->threads >= 4 ? 4 : c->threads >= 3 ? 3 : 2;
+    // last-level cache slows the callbacks' memcpy, and small batches pay the per-batch launch + copy latency.  A call over
+    // more devices than host slots therefore shares the host ring: every device gets device-side slots, and those beyond
+    // the first `base_slots` borrow the pinned buffers of slot i % base_slots (ZSTDMT_B200_NO_RING_SHARE=1: every slot its
+    // own, 8 x 8 MiB over 8 devices, 14.3 GB/s).
+    if (!ctx_devices(c)) return E.library;
+    const size_t base_slots = host_slots(c);
     size_t nsl = env_size("ZSTDMT_B200_SLOTS", base_slots > c->devs.size() ? base_slots : c->devs.size());
-    if (nsl < 2) nsl = 2; if (nsl < c->devs.size()) nsl = c->devs.size(); if (nsl > 64) nsl = 64;
-    size_t batch_bytes = env_size("ZSTDMT_B200_BATCH_MB", 8) << 20;
-    const bool no_alias = getenv("ZSTDMT_B200_NO_RING_SHARE") != nullptr;          // A/B knob: every slot its own pinned buffers
+    if (nsl < 2) nsl = 2;
+    if (nsl < c->devs.size()) nsl = c->devs.size();
+    if (nsl > 64) nsl = 64;
+    const bool no_alias = getenv("ZSTDMT_B200_NO_RING_SHARE") != nullptr;
     if (!no_alias && nsl > base_slots) nsl = (nsl + base_slots - 1) / base_slots * base_slots;   // batch q uses host buffer q % base_slots: needs base_slots | slots
-    size_t B = batch_bytes / chunk; if (B < 1) B = 1; if (B > 65536) B = 65536;
+    size_t B = (env_size("ZSTDMT_B200_BATCH_MB", 8) << 20) / chunk;
+    if (B < 1) B = 1;
+    if (B > 65536) B = 65536;
 
     if (P.slots.empty()) {
         P.slots.resize(nsl);
+        SlotCaps caps;
+        caps.in = B * chunk; caps.out = (size_t)ops->c_bound((uint32_t)B, (uint32_t)chunk); caps.work = ops->c_work((uint32_t)B, (uint32_t)chunk); caps.tab = B;
         for (size_t i = 0; i < P.slots.size(); i++) {
-            const size_t ic = B * chunk, oc = (size_t)ops->c_bound((uint32_t)B, (uint32_t)chunk), wc = ops->c_work((uint32_t)B, (uint32_t)chunk);
-            const bool okk = (i < base_slots || no_alias) ? slot_alloc(P.slots[i], c->devs[i % c->devs.size()], ic, oc, wc, B)
-                                                          : slot_alloc_alias(P.slots[i], P.slots[i % base_slots], c->devs[i % c->devs.size()], ic, oc, wc, B);
-            if (!okk) { ctx_release_slots(c); return E.mem; }
+            const Slot* owner = (i < base_slots || no_alias) ? nullptr : &P.slots[i % base_slots];
+            if (!slot_acquire(P.slots[i], c->devs[i % c->devs.size()], caps, owner)) { ctx_release_slots(c); return E.mem; }
         }
     }
     const size_t N = P.slots.size();
-    // batches in flight: slots beyond the first `base_slots` borrow their pinned buffers from slot i % base_slots, so batch q + H
-    // may only be filled once batch q has been written
-    const size_t H = (N > base_slots && !no_alias) ? base_slots : N;
-    P.fill_seq = P.submit_seq = P.write_seq = 0; P.reader_done = false; P.error = 0;
-    for (auto& s : P.slots) s.state = 0;
+    const size_t in_flight = (N > base_slots && !no_alias) ? base_slots : N;
 
-    // ---- reader: fills slots in sequence order (pt_compress read section, lz4-mt_compress.c:255-277)
-    StageClock ck_r, ck_w, ck_s;
-    const CpuSet host_cpus = common_local_cpus(c->devs);
-    std::thread reader([&]() {
-        const ScopedAffinity bind(host_cpus);
-        size_t frames_read = 0; bool eof = false;
-        while (!eof) {
-            Slot* s;
-            {
-                const double t0 = StageClock::now();
-                std::unique_lock<std::mutex> lk(P.mu);
-                s = &P.slots[P.fill_seq % N];
-                P.cv.wait(lk, [&] { return (s->state == 0 && P.fill_seq - P.write_seq < H) || P.error; });
-                ck_r.wait += StageClock::now() - t0;
-                if (P.error) break;
-            }
-            Tables T = tables_at(s->h_tab, s->tab_cap);
-            uint32_t n = 0; size_t got_bytes = 0;
-            while (n < B) {
-                GenBuffer b; b.buf = s->h_in + (size_t)n * chunk; b.size = chunk; b.allocated = chunk;
-                const double t0 = StageClock::now();
-                int rv = rw->fn_read(rw->arg_read, &b);
-                ck_r.cb += StageClock::now() - t0;
-                if (rv != 0) { P.fail(mt_error(E, rv)); eof = true; n = 0; break; }
-                if (b.size > chunk) { P.fail(E.read_fail); eof = true; n = 0; break; }
-                if (b.size == 0 && frames_read > 0) { eof = true; break; }
-                T.d[n] = (uint32_t)b.size; got_bytes += b.size; frames_read++; n++;
-            }
-            if (n == 0) break;
-            s->n = n; s->in_used = got_bytes;
-            {
-                std::lock_guard<std::mutex> g(P.mu);
-                c->insize += got_bytes; c->frames += n;
-                s->state = 1; P.fill_seq++;
-            }
-            P.cv.notify_all();
+    // reader: B chunks per slot (pt_compress read section, lz4-mt_compress.c:255-277)
+    size_t frames_read = 0;
+    auto fill = [&](Slot& s, bool& last) -> size_t {
+        const Tables T = tables_at(s.h_tab, s.cap.tab);
+        uint32_t n = 0; size_t got_bytes = 0;
+        while (n < B) {
+            size_t got = 0;
+            const size_t e = read_some(c, rw, s.h_in + (size_t)n * chunk, chunk, &got);
+            if (e) return e;
+            if (got == 0 && frames_read > 0) { last = true; break; }
+            T.frame_len[n] = (uint32_t)got; got_bytes += got; frames_read++; n++;
         }
-        { std::lock_guard<std::mutex> g(P.mu); P.reader_done = true; }
-        P.cv.notify_all();
-    });
-
-    // ---- writer: in-order emission (pt_write, lz4-mt_compress.c:178-205)
-    std::thread writer([&]() {
-        const ScopedAffinity bind(host_cpus);
-        for (;;) {
-            Slot* s;
-            {
-                const double t0 = StageClock::now();
-                std::unique_lock<std::mutex> lk(P.mu);
-                s = &P.slots[P.write_seq % N];
-                P.cv.wait(lk, [&] { return s->state == 2 || P.error || (P.reader_done && P.write_seq == P.fill_seq); });
-                ck_w.wait += StageClock::now() - t0;
-                if (P.error || s->state != 2) break;
-            }
-            cudaSetDevice(s->dev);
-            const double tg = StageClock::now();
-            if (cudaEventSynchronize(s->ev) != cudaSuccess) { c->lib_errcode = ZMT_ST_CUDA; P.fail(E.library); break; }
-            Tables T = tables_at(s->h_tab, s->tab_cap);
-            const uint64_t total = T.a[s->n];
-            if (total > s->out_cap) { c->lib_errcode = ZMT_ST_DST_SMALL; P.fail(E.library); break; }
-            if (cudaMemcpyAsync(s->h_out, s->d_out, total, cudaMemcpyDeviceToHost, s->stream) != cudaSuccess ||
-                cudaStreamSynchronize(s->stream) != cudaSuccess) { c->lib_errcode = ZMT_ST_CUDA; P.fail(E.library); break; }
-            ck_w.gpu += StageClock::now() - tg;
-            bool bad = false;
-            const double tc = StageClock::now();
-            for (uint32_t i = 0; i < s->n; i++) {
-                GenBuffer b; b.buf = s->h_out + T.a[i]; b.size = (size_t)(T.a[i + 1] - T.a[i]); b.allocated = b.size;
-                int rv = rw->fn_write(rw->arg_write, &b);
-                if (rv != 0) { P.fail(mt_error(E, rv)); bad = true; break; }
-                c->outsize += b.size; c->curframe++;
-            }
-            ck_w.cb += StageClock::now() - tc;
-            if (bad) break;
-            { std::lock_guard<std::mutex> g(P.mu); s->state = 0; P.write_seq++; }
-            P.cv.notify_all();
-        }
-    });
-
-    // ---- submit (calling thread)
-    for (;;) {
-        Slot* s;
-        {
-            const double t0 = StageClock::now();
-            std::unique_lock<std::mutex> lk(P.mu);
-            s = &P.slots[P.submit_seq % N];
-            P.cv.wait(lk, [&] { return s->state == 1 || P.error || (P.reader_done && P.submit_seq == P.fill_seq); });
-            ck_s.wait += StageClock::now() - t0;
-            if (P.error || s->state != 1) break;
-        }
-        const double ts = StageClock::now();
-        cudaSetDevice(s->dev);
-        Tables Th = tables_at(s->h_tab, s->tab_cap), Td = tables_at(s->d_tab, s->tab_cap);
+        s.n = n; s.in_used = got_bytes;
+        c->insize += got_bytes; c->frames += n;
+        return 0;
+    };
+    auto submit = [&](Slot& s) -> size_t {
+        const Tables Th = tables_at(s.h_tab, s.cap.tab), Td = tables_at(s.d_tab, s.cap.tab);
         bool full = true;
-        for (uint32_t i = 0; i < s->n; i++) if (Th.d[i] != chunk) { full = false; break; }
+        for (uint32_t i = 0; i < s.n; i++) if (Th.frame_len[i] != chunk) { full = false; break; }
         cudaError_t ce = cudaSuccess;
-        if (full) ce = cudaMemcpyAsync(s->d_in, s->h_in, (size_t)s->n * chunk, cudaMemcpyHostToDevice, s->stream);
-        else for (uint32_t i = 0; i < s->n && ce == cudaSuccess; i++)
-            if (Th.d[i]) ce = cudaMemcpyAsync(s->d_in + (size_t)i * chunk, s->h_in + (size_t)i * chunk, Th.d[i], cudaMemcpyHostToDevice, s->stream);
-        if (ce == cudaSuccess) ce = cudaMemcpyAsync(Td.d, Th.d, (size_t)s->n * 4, cudaMemcpyHostToDevice, s->stream);
+        if (full) ce = cudaMemcpyAsync(s.d_in, s.h_in, (size_t)s.n * chunk, cudaMemcpyHostToDevice, s.stream);
+        else for (uint32_t i = 0; i < s.n && ce == cudaSuccess; i++)
+            if (Th.frame_len[i]) ce = cudaMemcpyAsync(s.d_in + (size_t)i * chunk, s.h_in + (size_t)i * chunk, Th.frame_len[i], cudaMemcpyHostToDevice, s.stream);
+        if (ce == cudaSuccess) ce = cudaMemcpyAsync(Td.frame_len, Th.frame_len, (size_t)s.n * 4, cudaMemcpyHostToDevice, s.stream);
         int st = ZMT_ST_CUDA;
-        if (ce == cudaSuccess) st = ops->compress(s->d_in, 0, (uint32_t)chunk, Td.d, s->n, s->d_work, s->d_out, Td.a, s->stream);
-        if (s->dev >= 0 && s->dev < 64) g_dev_batches[s->dev]++;
+        if (ce == cudaSuccess) st = ops->compress(s.d_in, 0, (uint32_t)chunk, Td.frame_len, s.n, s.d_work, s.d_out, Td.out_off, s.stream);
         if (st == ZMT_ST_OK) {
-            ce = cudaMemcpyAsync(Th.a, Td.a, ((size_t)s->n + 1) * 8, cudaMemcpyDeviceToHost, s->stream);
-            if (ce == cudaSuccess) ce = cudaEventRecord(s->ev, s->stream);
+            ce = cudaMemcpyAsync(Th.out_off, Td.out_off, ((size_t)s.n + 1) * 8, cudaMemcpyDeviceToHost, s.stream);
+            if (ce == cudaSuccess) ce = cudaEventRecord(s.ev, s.stream);
             if (ce != cudaSuccess) st = ZMT_ST_CUDA;
         }
-        if (st != ZMT_ST_OK) { c->lib_errcode = (size_t)st; P.fail(E.library); break; }
-        ck_s.gpu += StageClock::now() - ts;
-        { std::lock_guard<std::mutex> g(P.mu); s->state = 2; P.submit_seq++; }
-        P.cv.notify_all();
-    }
-    reader.join(); writer.join();
-    for (auto& s : P.slots) { cudaSetDevice(s.dev); cudaStreamSynchronize(s.stream); }
-    if (trace_on())
-        fprintf(stderr, "[zstdmt_b200] compress: reader cb %.3fs wait %.3fs | submit enqueue %.3fs wait %.3fs | writer gpu-wait %.3fs cb %.3fs wait %.3fs | slots %zu x %zu chunks\n",
-                ck_r.cb, ck_r.wait, ck_s.gpu, ck_s.wait, ck_w.gpu, ck_w.cb, ck_w.wait, N, B);
-    return P.error;
+        if (st != ZMT_ST_OK) { c->lib_errcode = (size_t)st; return E.library; }
+        return 0;
+    };
+    // writer: one fn_write per frame, in order (pt_write, lz4-mt_compress.c:178-205)
+    auto drain = [&](Slot& s) -> size_t {
+        const Tables T = tables_at(s.h_tab, s.cap.tab);
+        const uint64_t total = T.out_off[s.n];
+        if (total > s.cap.out) { c->lib_errcode = ZMT_ST_DST_SMALL; return E.library; }
+        cudaError_t ce;
+        {
+            const Timed t(P.clk.wr_gpu);
+            ce = cudaMemcpyAsync(s.h_out, s.d_out, total, cudaMemcpyDeviceToHost, s.stream);
+            if (ce == cudaSuccess) ce = cudaStreamSynchronize(s.stream);
+        }
+        if (ce != cudaSuccess) { c->lib_errcode = ZMT_ST_CUDA; return E.library; }
+        for (uint32_t i = 0; i < s.n; i++) {
+            const size_t e = write_all(c, rw, s.h_out + T.out_off[i], (size_t)(T.out_off[i + 1] - T.out_off[i]));
+            if (e) return e;
+            c->curframe++;
+        }
+        return 0;
+    };
+    return run_pipeline(c, in_flight, fill, submit, drain);
 }
 
 // ------------------------------------------------------------------ decompression
+// Walks the block headers of the LZ4 frame p[0..n) (magic, FLG and BD already read): *bound = the sum of the blocks'
+// output bounds (each block <= blockMaxSize).  Returns the offset just past the end mark, 0 if the frame runs past n.
+size_t lz4f_walk_blocks(const uint8_t* p, size_t n, uint64_t* bound)
+{
+    const uint32_t flg = p[4], id = (p[5] >> 4) & 7;
+    const uint64_t blkmax = 1ull << (8 + 2 * id);
+    size_t q = 4 + 2 + ((flg & 8) ? 8 : 0) + ((flg & 1) ? 4 : 0) + 1;
+    *bound = 0;
+    for (;;) {
+        if (q + 4 > n) return 0;
+        const uint32_t bh = rd32(p + q); q += 4;
+        if (bh == 0) return q;
+        const uint32_t bs = bh & 0x7FFFFFFFu;
+        *bound += (bh & 0x80000000u) ? bs : blkmax;
+        q += (size_t)bs + ((flg & 0x10) ? 4 : 0);
+    }
+}
+
 // Output size of one payload, from its own header (pt_decompress sizes the buffer from
-// LE64 @ payload+6, lz4-mt_decompress.c:329-335; zstd: frame content size).
-// Returns false if the header is unusable.
+// LE64 @ payload+6, lz4-mt_decompress.c:329-335).  Returns false if the header is unusable.
 bool lz4f_out_size(const uint8_t* p, size_t n, uint64_t* out)
 {
     if (n < 7 || rd32(p) != LZ4F_MAGIC) { *out = 0; return true; }     // the device decoder reports the precise status
@@ -581,28 +607,22 @@ bool lz4f_out_size(const uint8_t* p, size_t n, uint64_t* out)
         if (v > (uint64_t)n * 255 + 65536) return false;
         *out = v; return true;
     }
-    // no content-size field: bound it by walking the block headers (each block <= blockMaxSize)
-    const uint32_t id = (bd >> 4) & 7; if (id < 4) return false;
-    const uint64_t blkmax = 1ull << (8 + 2 * id);
-    size_t pos = 4 + 2 + ((flg & 1) ? 4 : 0) + 1; uint64_t total = 0;
-    while (pos + 4 <= n) {
-        const uint32_t bh = rd32(p + pos); pos += 4;
-        if (bh == 0) break;
-        const uint32_t bs = bh & 0x7FFFFFFFu;
-        total += (bh & 0x80000000u) ? bs : blkmax;
-        pos += (size_t)bs + ((flg & 0x10) ? 4 : 0);
-    }
-    *out = total; return true;
+    if (((bd >> 4) & 7) < 4) return false;
+    lz4f_walk_blocks(p, n, out);                                         // no content-size field: the block walk bounds it
+    return true;
 }
 
-// reads exactly `want` bytes unless EOF; returns 0 ok / error; *got = delivered
-size_t read_some(const ErrCodes& E, GenRdWr* rw, void* dst, size_t want, size_t* got)
+// zstd / lz4 decode of one batch whose tables are on the device
+int launch_decode(bool is_zstd, const void* d_in, uint64_t in_bytes, const void* d_blk, uint32_t nblk, const Tables& Td, uint32_t n,
+                  uint32_t nslots, void* d_out, void* d_work, cudaStream_t st)
 {
-    GenBuffer b; b.buf = dst; b.size = want; b.allocated = want;
-    int rv = rw->fn_read(rw->arg_read, &b);
-    if (rv != 0) return mt_error(E, rv);
-    if (b.size > want) return E.read_fail;
-    *got = b.size; return 0;
+    return is_zstd ? zmt_zstd_decompress_device(d_in, d_blk, nblk, Td.first_blk, Td.expect, Td.frame_flags, n, d_out, Td.out_off, Td.out_size, Td.status, d_work, st)
+                   : zmt_lz4_decompress_device(d_in, in_bytes, Td.frame_off, Td.frame_len, n, nslots, d_out, Td.out_off, Td.out_size, Td.status, d_work, st);
+}
+
+size_t decode_work_bytes(bool is_zstd, const SlotCaps& k)
+{
+    return is_zstd ? zmt_zstdd_workspace_bytes((uint32_t)k.tab, k.blk, k.scr) : zmt_lz4d_workspace_bytes((uint32_t)k.tab, lz4_slot_cap(k.out, k.tab), k.in);
 }
 
 // ------------------------------------------------------------------ plain (unframed) single streams
@@ -649,7 +669,7 @@ size_t decompress_single_stream(Ctx* c, GenRdWr* rw, const uint8_t* first, size_
     for (;;) {
         // ---- cut complete frames out of what we hold, up to one batch
         foff.clear(); ooff.assign(1, 0); expect.clear(); fcs.clear(); first_blk.assign(1, 0); fflags.clear();
-        uint32_t nblk = 0; uint64_t scratch = 0, nslots = 0;
+        uint32_t nblk = 0, nslots = 0; uint64_t scratch = 0;
         const size_t batch_start = pos;
         bool need_more = false;
         while (!need_more) {
@@ -665,26 +685,17 @@ size_t decompress_single_stream(Ctx* c, GenRdWr* rw, const uint8_t* first, size_
             if (!is_zstd) {
                 if (magic != LZ4F_MAGIC) return E.data_error;
                 if (n - pos < 7) { if (eof) return E.data_error; need_more = true; break; }
-                const uint32_t flg = s[pos + 4], bd = s[pos + 5], id = (bd >> 4) & 7;
+                const uint32_t flg = s[pos + 4], id = (s[pos + 5] >> 4) & 7;
                 if ((flg >> 6) != 1 || id < 4) { c->lib_errcode = ZMT_ST_BAD_HEADER; return E.library; }
-                const uint64_t blkmax = 1ull << (8 + 2 * id);
-                size_t q = pos + 4 + 2 + ((flg & 8) ? 8 : 0) + ((flg & 1) ? 4 : 0) + 1;
-                uint64_t bound = 0; bool cut = false;
-                for (;;) {
-                    if (q + 4 > n) { cut = true; break; }
-                    const uint32_t bh = rd32(s + q); q += 4;
-                    if (bh == 0) break;
-                    const uint32_t bs = bh & 0x7FFFFFFFu;
-                    bound += (bh & 0x80000000u) ? bs : blkmax;
-                    q += (size_t)bs + ((flg & 0x10) ? 4 : 0);
-                }
-                if (!cut && (flg & 4)) q += 4;
-                if (cut || q > n) { if (eof) { c->lib_errcode = ZMT_ST_TRUNCATED; return E.frame_decompress; } need_more = true; break; }
+                uint64_t bound = 0;
+                size_t q = lz4f_walk_blocks(s + pos, n - pos, &bound);
+                if (q && (flg & 4)) q += 4;
+                if (!q || q > n - pos) { if (eof) return status_error(c, ZMT_ST_TRUNCATED); need_more = true; break; }
                 uint64_t osz = bound;
                 if (flg & 8) { osz = rd64(s + pos + 6); if (osz > bound) { c->lib_errcode = ZMT_ST_CONTENT_SIZE; return E.library; } }    // untrusted field, bounded by the block walk
-                foff.push_back(pos); fcs.push_back((uint32_t)(q - pos)); ooff.push_back(ooff.back() + osz);
-                { const uint64_t nb = (osz + 65535) / 65536; nslots += nb ? nb : 1; }
-                pos = q;
+                foff.push_back(pos); fcs.push_back((uint32_t)q); ooff.push_back(ooff.back() + osz);
+                nslots += lz4_block_slots(osz);
+                pos += q;
             } else {
                 if (magic < 0xFD2FB522u || magic > 0xFD2FB528u) return E.data_error;
                 uint64_t cs = 0; uint32_t fl = 0; size_t used = 0;
@@ -697,7 +708,7 @@ size_t decompress_single_stream(Ctx* c, GenRdWr* rw, const uint8_t* first, size_
                     blocks.resize(blocks.size() * 2 + 4096 * dsz);            // block table full: grow and rescan this frame
                 }
                 if (zr == ZMT_ST_TRUNCATED && !eof) { nblk = nblk0; scratch = scr0; need_more = true; break; }
-                if (zr != ZMT_ST_OK) { c->lib_errcode = (size_t)zr; return zr == ZMT_ST_TRUNCATED ? E.frame_decompress : E.library; }
+                if (zr != ZMT_ST_OK) return status_error(c, zr);
                 foff.push_back(pos); expect.push_back((fl & 4u) ? ~0ull : cs); fflags.push_back(fl); first_blk.push_back(nblk); ooff.push_back(ooff.back() + cs);
                 pos += used;
             }
@@ -711,39 +722,39 @@ size_t decompress_single_stream(Ctx* c, GenRdWr* rw, const uint8_t* first, size_
             const size_t in_bytes = pos + 12;                                   // frames address the buffer from its 12-byte pad
             const size_t tab_bytes = tables_bytes(nf);
             h_tab.resize(tab_bytes);
-            Tables T = tables_at(h_tab.data(), nf);
-            for (uint32_t i = 0; i < nf; i++) { T.a[i] = foff[i]; T.b[i] = ooff[i]; if (is_zstd) { T.f[i] = expect[i]; T.d[i] = fflags[i]; T.g[i] = first_blk[i]; } else T.d[i] = fcs[i]; }
-            T.b[nf] = total; if (is_zstd) T.g[nf] = nblk;
-            const size_t wk = is_zstd ? zmt_zstdd_workspace_bytes(nf, nblk, scratch) : zmt_lz4d_workspace_bytes(nf, (uint32_t)nslots, in_bytes);
+            const Tables T = tables_at(h_tab.data(), nf);
+            for (uint32_t i = 0; i < nf; i++) {
+                T.frame_off[i] = foff[i]; T.out_off[i] = ooff[i];
+                if (is_zstd) { T.expect[i] = expect[i]; T.frame_flags[i] = fflags[i]; T.first_blk[i] = first_blk[i]; } else T.frame_len[i] = fcs[i];
+            }
+            T.out_off[nf] = total; if (is_zstd) T.first_blk[nf] = nblk;
+            const size_t wk = is_zstd ? zmt_zstdd_workspace_bytes(nf, nblk, scratch) : zmt_lz4d_workspace_bytes(nf, nslots, in_bytes);
             if (!d_in.need(in_bytes + 256) || !d_out.need(total + 256) || !d_tab.need(tab_bytes) || !d_work.need(wk) || (is_zstd && !d_blk.need((size_t)nblk * dsz + 16))) return E.mem;
-            Tables Td = tables_at((uint8_t*)d_tab.p, nf);
+            const Tables Td = tables_at((uint8_t*)d_tab.p, nf);
             // only the bytes of this batch travel (the device addresses them at their buffer offsets)
             const size_t lo = 12 + batch_start, hi = in_bytes;
             cudaMemcpyAsync((uint8_t*)d_in.p + lo, in.data() + lo, hi - lo, cudaMemcpyHostToDevice, st);
             cudaMemcpyAsync(d_tab.p, h_tab.data(), tab_bytes, cudaMemcpyHostToDevice, st);
             if (is_zstd && nblk) cudaMemcpyAsync(d_blk.p, blocks.data(), (size_t)nblk * dsz, cudaMemcpyHostToDevice, st);
-            const int rc = is_zstd ? zmt_zstd_decompress_device(d_in.p, d_blk.p, nblk, Td.g, Td.f, Td.d, nf, d_out.p, Td.b, Td.c, Td.e, d_work.p, st)
-                                   : zmt_lz4_decompress_device(d_in.p, in_bytes, Td.a, Td.d, nf, (uint32_t)nslots, d_out.p, Td.b, Td.c, Td.e, d_work.p, st);
+            const int rc = launch_decode(is_zstd, d_in.p, in_bytes, d_blk.p, nblk, Td, nf, nslots, d_out.p, d_work.p, st);
             out.resize(total ? total : 1);
             std::vector<uint32_t> status(nf); std::vector<uint64_t> osz(nf);
             cudaError_t ce = cudaSuccess;
             if (rc == ZMT_ST_OK) {
                 if (total) ce = cudaMemcpyAsync(out.data(), d_out.p, total, cudaMemcpyDeviceToHost, st);
-                if (ce == cudaSuccess) ce = cudaMemcpyAsync(status.data(), Td.e, (size_t)nf * 4, cudaMemcpyDeviceToHost, st);
-                if (ce == cudaSuccess) ce = cudaMemcpyAsync(osz.data(), Td.c, (size_t)nf * 8, cudaMemcpyDeviceToHost, st);
+                if (ce == cudaSuccess) ce = cudaMemcpyAsync(status.data(), Td.status, (size_t)nf * 4, cudaMemcpyDeviceToHost, st);
+                if (ce == cudaSuccess) ce = cudaMemcpyAsync(osz.data(), Td.out_size, (size_t)nf * 8, cudaMemcpyDeviceToHost, st);
                 if (ce == cudaSuccess) ce = cudaStreamSynchronize(st);
             }
             if (rc != ZMT_ST_OK || ce != cudaSuccess) { cudaGetLastError(); c->lib_errcode = ZMT_ST_CUDA; return E.library; }
             for (uint32_t i = 0; i < nf; i++) {
-                if (status[i] != ZMT_ST_OK) { c->lib_errcode = status[i]; return (status[i] == ZMT_ST_TRUNCATED || status[i] == ZMT_ST_TRAILING) ? E.frame_decompress : E.library; }
+                if (status[i] != ZMT_ST_OK) return status_error(c, status[i]);
                 // frame by frame, in pieces of at most `piece` bytes (st_decompress writes as it goes)
-                uint64_t o = 0;
-                while (o < osz[i]) {
-                    GenBuffer b; b.buf = out.data() + ooff[i] + o; b.size = (size_t)((osz[i] - o) < piece ? (osz[i] - o) : piece); b.allocated = b.size;
-                    const size_t want = b.size;
-                    const int rv = rw->fn_write(rw->arg_write, &b);
-                    if (rv != 0) return mt_error(E, rv);
-                    c->outsize += b.size; o += want;
+                for (uint64_t o = 0; o < osz[i];) {
+                    const size_t len = (size_t)((osz[i] - o) < piece ? (osz[i] - o) : piece);
+                    const size_t e = write_all(c, rw, out.data() + ooff[i] + o, len);
+                    if (e) return e;
+                    o += len;
                 }
             }
             // drop what has been decoded
@@ -759,7 +770,7 @@ size_t decompress_single_stream(Ctx* c, GenRdWr* rw, const uint8_t* first, size_
                 const size_t old = in.size();
                 in.resize(old + piece);
                 size_t got = 0;
-                const size_t e = read_some(E, rw, in.data() + old, piece, &got);
+                const size_t e = read_some(c, rw, in.data() + old, piece, &got);
                 in.resize(old + got);
                 if (e) return e;
                 c->insize += got;
@@ -770,326 +781,283 @@ size_t decompress_single_stream(Ctx* c, GenRdWr* rw, const uint8_t* first, size_
     return 0;
 }
 
-size_t decompress_run(Ctx* c, GenRdWr* rw)
-{
-    const DeviceRestore restore_device;
-    const ErrCodes& E = *c->E;
-    Pipe& P = c->pipe;
-    const bool is_zstd = c->codec == CODEC_ZSTD;
-    const uint32_t kBlkCap = 32768;
-    // decode batches must hold enough frames to fill the GPU (one warp per 64 KiB block): 32 MiB of frames measured best
-    const size_t in_cap0 = (env_size("ZSTDMT_B200_DBATCH_MB", 32) << 20), out_cap0 = in_cap0 * 2, tab_cap = 8192;
-    const uint64_t piece_bytes = (uint64_t)env_size("ZSTDMT_B200_D2H_PIECE_MB", 2) << 20;      // 0: whole slot right after the kernels (measured 0 / 2 / 4 / 8 MiB: 12.8 / 15.1 / 14.3 / 12.8 GB/s)
+// ---- framed streams: the pipeline
+// What the reader has put into one decompress slot so far.
+struct BatchFill {
+    uint32_t n = 0, nblk = 0, nslots = 0;
+    size_t in_used = 0;
+    uint64_t out_used = 0, scr = 0;
+    SlotCaps need;                      // after ADMIT_MOVE: what a slot holding this frame alone needs
+};
+enum Admit { ADMIT_APPEND, ADMIT_MOVE, ADMIT_ERROR };
 
-    // ---- stream-type sniffing on the calling thread (LZ4MT_decompressDCtx, lz4-mt_decompress.c:503-520;
-    //      ZSTDCB_decompressDCtx, zstd-mt_decompress.c:721-759)
-    uint8_t first[16]; size_t have = 0, got = 0;
-    bool hdr_pending = false;                 // first 12-byte header already (partly) read into `first`
-    size_t first_payload_have = 0;            // zstd pzstd-style: 4 payload bytes already read
-    if (c->codec == CODEC_LZ4) {
-        size_t e = read_some(E, rw, first, 4, &got); if (e) return e;
+// Sizes the frame (12-byte header + `len` payload bytes) at s.h_in + bf.in_used — LZ4 from its header, zstd by the host
+// block scan — and appends it to the batch tables, or reports that it does not fit behind the frames already in the
+// slot (ADMIT_MOVE) or that it is broken (ADMIT_ERROR, *err = the call's error).
+Admit admit_frame(Ctx* c, Slot& s, BatchFill& bf, uint32_t len, size_t* err)
+{
+    const bool is_zstd = c->codec == CODEC_ZSTD;
+    const uint8_t* p = s.h_in + bf.in_used + 12;
+    uint64_t osz = 0, scr = bf.scr;
+    uint32_t flags = 0, nblk = bf.nblk;
+    bool fits = true;
+    bf.need = SlotCaps();
+    if (!is_zstd) {
+        if (!lz4f_out_size(p, len, &osz)) { c->lib_errcode = ZMT_ST_BAD_HEADER; *err = c->E->library; return ADMIT_ERROR; }
+    } else {
+        int zr;
+        { const Timed t(c->pipe.clk.rd_scan); zr = zmt_zstd_scan_frame_host(p, len, bf.in_used + 12, bf.n, s.h_blk, &nblk, s.cap.blk, &scr, &osz, &flags); }
+        if (zr == ZMT_ST_DST_SMALL) { fits = false; bf.need.blk = len / 3 + 16; }       // more blocks than descriptors: every block costs >= 3 bytes
+        else if (zr != ZMT_ST_OK) { *err = status_error(c, zr); return ADMIT_ERROR; }
+        else if (scr > s.cap.scr) fits = false;
+    }
+    if (fits && osz > s.cap.out - bf.out_used) fits = false;
+    if (!fits) { bf.need.in = 12 + (size_t)len; bf.need.out = osz; bf.need.scr = scr; return ADMIT_MOVE; }
+    const Tables T = tables_at(s.h_tab, s.cap.tab);
+    T.frame_off[bf.n] = bf.in_used; T.frame_len[bf.n] = len; T.out_off[bf.n] = bf.out_used;
+    if (is_zstd) { T.first_blk[bf.n] = bf.nblk; T.expect[bf.n] = (flags & 4u) ? ~0ull : osz; T.frame_flags[bf.n] = flags; bf.nblk = nblk; bf.scr = scr; }   // flag 4: no content size in the header, osz is a bound
+    else bf.nslots += lz4_block_slots(osz);
+    bf.in_used += 12 + (size_t)len; bf.out_used += osz; bf.n++;
+    return ADMIT_APPEND;
+}
+
+// The reader of a framed decode (pt_read, lz4-mt_decompress.c:192-281 / zstd-mt_decompress.c:209-369): frames behind
+// 12-byte skippable headers, read on the reader thread into the slot of each batch.
+struct FramedReader {
+    Ctx* c; GenRdWr* rw; bool is_zstd;
+    uint8_t first[16];                   // what the stream-type sniffing read
+    bool hdr_pending = false;            // first 12-byte header already (partly) read into `first`
+    size_t first_payload_have = 0;       // zstd pzstd-style: 4 payload bytes already read
+    std::vector<uint8_t> carry;          // a whole frame that did not fit where it was read: it starts a batch
+    size_t stat_in = 0;                  // input bytes of the batch being filled (insize counts committed batches)
+
+    FramedReader(Ctx* c_, GenRdWr* rw_) : c(c_), rw(rw_), is_zstd(c_->codec == CODEC_ZSTD) {}
+    size_t sniff(bool* framed);
+    size_t fill(Slot& s, bool& last);
+    size_t read_frame(Slot& s, const BatchFill& bf, uint32_t* len, bool* eof);
+    size_t place(Slot& s, BatchFill& bf, uint32_t len, bool* moved);
+    bool grow(Slot& s, const SlotCaps& need);
+};
+
+// Stream-type sniffing on the calling thread (LZ4MT_decompressDCtx, lz4-mt_decompress.c:503-520; ZSTDCB_decompressDCtx,
+// zstd-mt_decompress.c:721-759).  A plain stream is decoded right here (*framed = false, the call's result returned).
+size_t FramedReader::sniff(bool* framed)
+{
+    const ErrCodes& E = *c->E;
+    size_t got = 0;
+    *framed = false;
+    if (!is_zstd) {
+        size_t e = read_some(c, rw, first, 4, &got); if (e) return e;
         if (got != 4) return E.data_error;
         if (rd32(first) != MT_MAGIC_SKIPPABLE) {
             if (rd32(first) != LZ4F_MAGIC) return E.data_error;
             return decompress_single_stream(c, rw, first, 4);          // plain .lz4 stream (st_decompress, lz4-mt_decompress.c:512-520)
         }
-        e = read_some(E, rw, first + 4, 8, &got); if (e) return e;
+        e = read_some(c, rw, first + 4, 8, &got); if (e) return e;
         if (got != 8) return E.read_fail;
-        have = 12; hdr_pending = true;
     } else {
-        size_t e = read_some(E, rw, first, 16, &got); if (e) return e;
-        have = got;
-        auto is_zstd = [](const uint8_t* p) { uint32_t m = rd32(p); return m >= 0xFD2FB522u && m <= 0xFD2FB528u; };
+        size_t e = read_some(c, rw, first, 16, &got); if (e) return e;
+        auto is_zstd_magic = [](const uint8_t* p) { uint32_t m = rd32(p); return m >= 0xFD2FB522u && m <= 0xFD2FB528u; };
         auto is_skip = [](const uint8_t* p) { return rd32(p) == MT_MAGIC_SKIPPABLE && rd32(p + 4) == 4; };
-        if (have < 16) {
-            if (have < 4 || !is_zstd(first)) return E.data_error;
-            if (have == 9) return 0;                                   // empty file (zstd-mt_decompress.c:735-740)
-            return decompress_single_stream(c, rw, first, have);       // short plain zstd stream
+        if (got < 16) {
+            if (got < 4 || !is_zstd_magic(first)) return E.data_error;
+            if (got == 9) return 0;                                    // empty file (zstd-mt_decompress.c:735-740)
+            return decompress_single_stream(c, rw, first, got);        // short plain zstd stream
         }
         c->insize += 16;
-        if (is_skip(first) && is_zstd(first + 12)) { hdr_pending = true; first_payload_have = 4; }          // pzstd style
-        else if (is_zstd(first) && rd32(first + 9) == MT_MAGIC_SKIPPABLE) {                                    // zstdmt style: 9-byte empty frame + 12-byte header
+        if (is_skip(first) && is_zstd_magic(first + 12)) first_payload_have = 4;                                // pzstd style
+        else if (is_zstd_magic(first) && rd32(first + 9) == MT_MAGIC_SKIPPABLE) {                                  // zstdmt style: 9-byte empty frame + 12-byte header
             // (only the magic can be tested here, as IsZstd_Skippable does, zstd-mt_decompress.c:156-159: 7 of the header's 12
             //  bytes are in hand; the size field is checked with the assembled header.  Round 1 read its 4 bytes past the buffer.)
             uint8_t tmp[12]; memcpy(tmp, first + 9, 7);
-            size_t e2 = read_some(E, rw, tmp + 7, 5, &got); if (e2) return e2;
+            e = read_some(c, rw, tmp + 7, 5, &got); if (e) return e;
             if (got != 5) return E.data_error;
-            c->insize += 5; memcpy(first, tmp, 12); hdr_pending = true; first_payload_have = 0;
-        } else if (is_zstd(first)) return decompress_single_stream(c, rw, first, have);    // plain .zst (zstd-mt_decompress.c:747-752)
+            c->insize += 5; memcpy(first, tmp, 12);
+        } else if (is_zstd_magic(first)) return decompress_single_stream(c, rw, first, 16);    // plain .zst (zstd-mt_decompress.c:747-752)
         else return E.data_error;
     }
+    hdr_pending = true; *framed = true;
+    return 0;
+}
 
+// One batch: frames until the slot's table is full, a frame does not fit (it starts the next batch) or the input ends.
+size_t FramedReader::fill(Slot& s, bool& last)
+{
+    BatchFill bf;
+    bool moved = false;
+    stat_in = 0;
+    while (bf.n < s.cap.tab && !moved) {
+        uint32_t len = 0;
+        if (carry.empty()) {
+            const size_t e = read_frame(s, bf, &len, &last);
+            if (e) return e;
+            if (last) break;
+        } else len = (uint32_t)(carry.size() - 12);
+        const size_t e = place(s, bf, len, &moved);
+        if (e) return e;
+    }
+    s.n = bf.n;
+    if (bf.n == 0) return 0;
+    const Tables T = tables_at(s.h_tab, s.cap.tab);
+    T.out_off[bf.n] = bf.out_used;
+    if (is_zstd) T.first_blk[bf.n] = bf.nblk;
+    s.nblk = bf.nblk; s.nslots = bf.nslots; s.in_used = bf.in_used; s.out_used = (size_t)bf.out_used;
+    c->insize += stat_in; c->frames += bf.n;
+    return 0;
+}
+
+// The next frame of the input: read behind the frames already in the slot if it fits there, else into `carry`.
+// *eof at the end of the input.
+size_t FramedReader::read_frame(Slot& s, const BatchFill& bf, uint32_t* len, bool* eof)
+{
+    const ErrCodes& E = *c->E;
+    uint8_t hdr[12]; size_t pre = 0, g = 0;
+    if (hdr_pending) { memcpy(hdr, first, 12); hdr_pending = false; pre = first_payload_have; }
+    else {
+        const size_t e = read_some(c, rw, hdr, 12, &g);
+        if (e) return e;
+        if (g == 0) { *eof = true; return 0; }
+        if (g != 12) return E.read_fail;
+        if (rd32(hdr) != MT_MAGIC_SKIPPABLE) return E.data_error;
+        if (is_zstd) stat_in += 12;
+    }
+    if (rd32(hdr + 4) != 4) return E.data_error;
+    if (!is_zstd) stat_in += 12;
+    *len = rd32(hdr + 8);
+    if (*len < pre) return E.data_error;
+    uint8_t* dst = s.h_in + bf.in_used;
+    if (bf.in_used + 12 + *len > s.cap.in) { carry.resize(12 + (size_t)*len); dst = carry.data(); }
+    memcpy(dst, hdr, 12);
+    if (pre) memcpy(dst + 12, first + 12, pre);
+    const size_t e = read_some(c, rw, dst + 12 + pre, *len - pre, &g);
+    if (e) return e;
+    if (g != *len - pre) return E.data_error;
+    stat_in += g;
+    return 0;
+}
+
+// Appends the frame held in `carry` (or already at s.h_in + bf.in_used when `carry` is empty) to the batch.  A frame
+// that does not fit behind the others stays in `carry` for the next batch (*moved); a single frame larger than the
+// slot grows the empty slot (input, output, zstd block table and entropy scratch) until it fits.
+size_t FramedReader::place(Slot& s, BatchFill& bf, uint32_t len, bool* moved)
+{
+    const size_t flen = 12 + (size_t)len;
+    for (int tries = 0;; tries++) {
+        if (!carry.empty()) {
+            if (bf.in_used + flen > s.cap.in) {
+                if (bf.n > 0) { *moved = true; return 0; }
+                SlotCaps need; need.in = flen;
+                if (!grow(s, need)) return c->E->mem;
+            }
+            memcpy(s.h_in + bf.in_used, carry.data(), flen);
+        }
+        size_t e = 0;
+        const Admit a = admit_frame(c, s, bf, len, &e);
+        if (a == ADMIT_ERROR) return e;
+        if (a == ADMIT_APPEND) { carry.clear(); return 0; }
+        if (carry.empty()) carry.assign(s.h_in + bf.in_used, s.h_in + bf.in_used + flen);
+        if (bf.n > 0) { *moved = true; return 0; }
+        if (tries == 2 || !grow(s, bf.need)) return c->E->mem;
+    }
+}
+
+// (Re)allocates the still empty slot with at least the capacities in `need`; under the pipeline's mutex because the
+// writer's wait reads s.state.
+bool FramedReader::grow(Slot& s, const SlotCaps& need)
+{
+    SlotCaps k = s.cap;
+    if (need.in > k.in) k.in = need.in;
+    if (need.out > k.out) k.out = need.out;
+    if (need.blk > k.blk) k.blk = need.blk;
+    k.scr = is_zstd ? (need.scr > 3 * (uint64_t)k.out ? need.scr : 3 * (uint64_t)k.out) : 0;
+    k.work = decode_work_bytes(is_zstd, k);
+    std::lock_guard<std::mutex> g(c->pipe.mu);
+    const int dev = s.dev;
+    slot_release(s);
+    return slot_acquire(s, dev, k, nullptr);
+}
+
+// Submit of a decode batch: H2D of the frames and tables, the decoder, D2H of sizes and status (and of the whole output
+// when piece_bytes is 0).
+size_t decode_submit(Ctx* c, Slot& s, uint64_t piece_bytes)
+{
+    const bool is_zstd = c->codec == CODEC_ZSTD;
+    const Tables Th = tables_at(s.h_tab, s.cap.tab), Td = tables_at(s.d_tab, s.cap.tab);
+    cudaError_t ce = cudaMemcpyAsync(s.d_in, s.h_in, s.in_used, cudaMemcpyHostToDevice, s.stream);
+    if (ce == cudaSuccess) ce = cudaMemcpyAsync(s.d_tab, s.h_tab, s.tab_bytes, cudaMemcpyHostToDevice, s.stream);
+    if (ce == cudaSuccess && is_zstd && s.nblk) ce = cudaMemcpyAsync(s.d_blk, s.h_blk, (size_t)s.nblk * zmt_zstd_blk_desc_bytes(), cudaMemcpyHostToDevice, s.stream);
+    int st = ZMT_ST_CUDA;
+    if (ce == cudaSuccess) st = launch_decode(is_zstd, s.d_in, s.in_used, s.d_blk, s.nblk, Td, s.n, s.nslots, s.d_out, s.d_work, s.stream);
+    if (st == ZMT_ST_OK) {
+        if (s.out_used && piece_bytes == 0) ce = cudaMemcpyAsync(s.h_out, s.d_out, s.out_used, cudaMemcpyDeviceToHost, s.stream);
+        if (ce == cudaSuccess) ce = cudaMemcpyAsync(Th.out_size, Td.out_size, (size_t)s.n * 8, cudaMemcpyDeviceToHost, s.stream);
+        if (ce == cudaSuccess) ce = cudaMemcpyAsync(Th.status, Td.status, (size_t)s.n * 4, cudaMemcpyDeviceToHost, s.stream);
+        if (ce == cudaSuccess) ce = cudaEventRecord(s.ev, s.stream);
+        if (ce != cudaSuccess) st = ZMT_ST_CUDA;
+    }
+    if (st != ZMT_ST_OK) { c->lib_errcode = (size_t)st; return c->E->library; }
+    return 0;
+}
+
+// Writer of a decode batch (pt_write, lz4-mt_decompress.c:165-187): one fn_write per frame.  The decoded bytes come over
+// in pieces of piece_bytes, one piece ahead of the one being written: what fn_write's memcpy reads was DMA-written
+// moments ago and is still in the last-level cache, instead of a whole 64 MiB slot that was copied long before its
+// first byte is used.
+size_t decode_drain(Ctx* c, GenRdWr* rw, Slot& s, uint64_t piece_bytes)
+{
+    const Tables T = tables_at(s.h_tab, s.cap.tab);
+    uint32_t issued = 0, ready = 0, piece_end[2] = { 0, 0 };     // frames [0, issued) requested, [0, ready) landed
+    int np_issued = 0, np_ready = 0;                               // piece k: event evp[k & 1], frames up to piece_end[k & 1]
+    auto issue_piece = [&]() -> bool {
+        uint32_t j = issued; const uint64_t lo = T.out_off[j]; uint64_t hi = lo;
+        while (j < s.n && hi - lo < piece_bytes) { hi = T.out_off[j] + T.out_size[j]; j++; }
+        if (hi > s.cap.out) hi = s.cap.out;
+        if (hi > lo && cudaMemcpyAsync(s.h_out + lo, s.d_out + lo, (size_t)(hi - lo), cudaMemcpyDeviceToHost, s.stream) != cudaSuccess) return false;
+        if (cudaEventRecord(s.evp[np_issued & 1], s.stream) != cudaSuccess) return false;
+        piece_end[np_issued++ & 1] = issued = j;
+        return true;
+    };
+    for (uint32_t i = 0; i < s.n; i++) {
+        if (T.status[i] != ZMT_ST_OK) return status_error(c, T.status[i]);
+        if (piece_bytes && i >= ready) {
+            bool ok = np_issued > np_ready || issue_piece();                                // the piece holding frame i
+            if (ok && issued < s.n && np_issued == np_ready + 1) ok = issue_piece();        // and one ahead
+            ok = ok && cudaEventSynchronize(s.evp[np_ready & 1]) == cudaSuccess;
+            if (!ok) { c->lib_errcode = ZMT_ST_CUDA; return c->E->library; }
+            ready = piece_end[np_ready++ & 1];
+        }
+        const size_t e = write_all(c, rw, s.h_out + T.out_off[i], (size_t)T.out_size[i]);
+        if (e) return e;
+        c->curframe++;
+    }
+    return 0;
+}
+
+size_t decompress_run(Ctx* c, GenRdWr* rw)
+{
+    const DeviceRestore restore_device;
+    Pipe& P = c->pipe;
+    const bool is_zstd = c->codec == CODEC_ZSTD;
+    FramedReader reader(c, rw);
+    bool framed = false;
+    const size_t r = reader.sniff(&framed);
+    if (!framed) return r;
+    if (!ctx_devices(c)) return c->E->library;
     if (P.slots.empty()) {
-        c->devs = env_devices();
-        if (c->devs.empty()) { c->lib_errcode = ZMT_ST_CUDA; return E.library; }
-        const size_t base_slots = c->threads >= 4 ? 4 : c->threads >= 3 ? 3 : 2;       // see compress_run
+        const size_t base_slots = host_slots(c);
         P.slots.resize(base_slots > c->devs.size() ? base_slots : c->devs.size());
+        // decode batches must hold enough frames to fill the GPU (one warp per 64 KiB block): 32 MiB of frames measured best
+        SlotCaps caps;
+        caps.in = env_size("ZSTDMT_B200_DBATCH_MB", 32) << 20; caps.out = 2 * caps.in; caps.tab = 8192;
+        // zstd scratch: 16 B per sequence + the literals: ~2x the output on text, bounded at 3x + tables (the reader closes a batch early otherwise)
+        if (is_zstd) { caps.blk = 32768; caps.scr = 3 * (uint64_t)caps.out; }
+        caps.work = decode_work_bytes(is_zstd, caps);
         for (size_t i = 0; i < P.slots.size(); i++)
-        {
-            // zstd scratch: 16 B per sequence + the literals: ~2x the output on text, bounded at 3x + tables (the reader closes a batch early otherwise)
-            const size_t wk = is_zstd ? zmt_zstdd_workspace_bytes((uint32_t)tab_cap, kBlkCap, 3 * (uint64_t)out_cap0) : zmt_lz4d_workspace_bytes((uint32_t)tab_cap, lz4_slot_cap(out_cap0, tab_cap), in_cap0);
-            if (!slot_alloc(P.slots[i], c->devs[i % c->devs.size()], in_cap0, out_cap0, wk, tab_cap) || (is_zstd && !slot_ensure_blocks(P.slots[i], kBlkCap))) { ctx_release_slots(c); return E.mem; }
-            P.slots[i].scr_cap = is_zstd ? 3 * (uint64_t)P.slots[i].out_cap : 0;
-        }
+            if (!slot_acquire(P.slots[i], c->devs[i % c->devs.size()], caps, nullptr)) { ctx_release_slots(c); return c->E->mem; }
     }
-    const size_t N = P.slots.size();
-    P.fill_seq = P.submit_seq = P.write_seq = 0; P.reader_done = false; P.error = 0;
-    for (auto& s : P.slots) s.state = 0;
-
-    StageClock rd_clk, wr_clk; double rd_scan = 0, rd_total = 0, wr_total = 0;     // ZSTDMT_B200_TRACE=1
-    const bool tr = trace_on();
-    // ---- reader (pt_read, lz4-mt_decompress.c:192-281 / zstd-mt_decompress.c:209-369)
-    const CpuSet host_cpus = common_local_cpus(c->devs);
-    std::thread reader([&]() {
-        const ScopedAffinity bind(host_cpus);
-        const double t_start = tr ? StageClock::now() : 0;
-        bool eof = false;
-        std::vector<uint8_t> carry;              // a frame that did not fit the previous slot
-        uint64_t carry_out = 0;
-        while (!eof) {
-            Slot* s;
-            {
-                std::unique_lock<std::mutex> lk(P.mu);
-                s = &P.slots[P.fill_seq % N];
-                const double t0 = tr ? StageClock::now() : 0;
-                P.cv.wait(lk, [&] { return s->state == 0 || P.error; });
-                if (tr) rd_clk.wait += StageClock::now() - t0;
-                if (P.error) break;
-            }
-            Tables T = tables_at(s->h_tab, s->tab_cap);
-            uint32_t n = 0; size_t in_used = 0; uint64_t out_used = 0; size_t stat_in = 0;
-            bool failed = false;
-            uint32_t nblk = 0; uint64_t scr = 0;                 // zstd: block descriptors + scratch demand of this batch
-            // (re)allocate the still empty slot so that one frame of these dimensions fits; takes P.mu for the swap because the
-            // writer's wait predicate reads s->state
-            auto grow = [&](size_t need_in, uint64_t need_out, uint64_t need_scr, uint32_t need_blk) -> bool {
-                if (need_in <= s->in_cap && need_out <= s->out_cap && need_scr <= s->scr_cap && need_blk <= s->blk_cap) return true;
-                const int dev = s->dev;
-                const size_t nin = need_in > s->in_cap ? need_in : s->in_cap, nout = need_out > s->out_cap ? (size_t)need_out : s->out_cap;
-                const uint64_t nscr = is_zstd ? (need_scr > 3 * (uint64_t)nout ? need_scr : 3 * (uint64_t)nout) : 0;
-                const uint32_t nb = need_blk > s->blk_cap ? need_blk : s->blk_cap;
-                const size_t tc = s->tab_cap;
-                const size_t wk = is_zstd ? zmt_zstdd_workspace_bytes((uint32_t)tc, nb, nscr) : zmt_lz4d_workspace_bytes((uint32_t)tc, lz4_slot_cap(nout, tc), nin);
-                std::lock_guard<std::mutex> g(P.mu);
-                slot_free(*s);
-                if (!slot_alloc(*s, dev, nin, nout, wk, tc) || (is_zstd && !slot_ensure_blocks(*s, nb))) return false;
-                s->scr_cap = nscr;
-                return true;
-            };
-            // Put one whole frame (12-byte header + payload, held in `fr`) at the start of the empty slot, growing the slot
-            // (input, output, zstd block table and entropy scratch) until it fits.  Returns false after P.fail().
-            auto place_first = [&](const std::vector<uint8_t>& fr) -> bool {
-                const size_t toRead = fr.size() - 12;
-                if (!grow(fr.size(), 0, 0, 0)) { P.fail(E.mem); return false; }
-                uint64_t osz = 0; uint32_t nsq = 0;
-                if (!is_zstd) {
-                    if (!lz4f_out_size(fr.data() + 12, toRead, &osz)) { c->lib_errcode = ZMT_ST_BAD_HEADER; P.fail(E.library); return false; }
-                    if (!grow(fr.size(), osz, 0, 0)) { P.fail(E.mem); return false; }
-                    memcpy(s->h_in, fr.data(), fr.size());
-                } else {
-                    for (int tries = 0;; tries++) {
-                        memcpy(s->h_in, fr.data(), fr.size());
-                        uint64_t cs = 0; nblk = 0; scr = 0;
-                        const int zr = zmt_zstd_scan_frame_host(s->h_in + 12, toRead, 12, 0, s->h_blk, &nblk, s->blk_cap, &scr, &cs, &nsq);
-                        if (zr == ZMT_ST_DST_SMALL && tries < 2) {          // more blocks than descriptors: every block costs >= 3 bytes
-                            if (!grow(fr.size(), 0, 0, (uint32_t)(toRead / 3 + 16))) { P.fail(E.mem); return false; }
-                            continue;
-                        }
-                        if (zr != ZMT_ST_OK) { c->lib_errcode = (size_t)zr; P.fail(zr == ZMT_ST_TRUNCATED || zr == ZMT_ST_TRAILING ? E.frame_decompress : E.library); return false; }
-                        osz = cs;
-                        if (osz <= s->out_cap && scr <= s->scr_cap) break;
-                        if (tries >= 2 || !grow(fr.size(), osz, scr, 0)) { P.fail(E.mem); return false; }
-                    }
-                }
-                T = tables_at(s->h_tab, s->tab_cap);
-                T.a[0] = 0; T.d[0] = (uint32_t)toRead; T.b[0] = 0;
-                if (is_zstd) { T.g[0] = 0; T.f[0] = (nsq & 4u) ? ~0ull : osz; T.d[0] = nsq; }      // flag 4: no content size in the header, osz is a bound
-                in_used = fr.size(); out_used = osz; n = 1;
-                return true;
-            };
-            if (!carry.empty()) {
-                if (!place_first(carry)) break;
-                carry.clear();
-            }
-            while (n < s->tab_cap) {
-                uint8_t hdr[12]; size_t pre = 0;
-                if (hdr_pending) { memcpy(hdr, first, 12); hdr_pending = false; pre = first_payload_have; }
-                else {
-                    size_t g = 0; size_t e = read_some(E, rw, hdr, 12, &g);
-                    if (e) { P.fail(e); failed = true; break; }
-                    if (g == 0) { eof = true; break; }
-                    if (g != 12) { P.fail(E.read_fail); failed = true; break; }
-                    if (rd32(hdr) != MT_MAGIC_SKIPPABLE) { P.fail(E.data_error); failed = true; break; }
-                    if (c->codec == CODEC_ZSTD) stat_in += 12;
-                }
-                if (rd32(hdr + 4) != 4) { P.fail(E.data_error); failed = true; break; }
-                if (c->codec == CODEC_LZ4) stat_in += 12;
-                const size_t toRead = rd32(hdr + 8);
-                if (toRead < pre) { P.fail(E.data_error); failed = true; break; }
-                // where to put it: the current slot if it fits behind the frames already there, else a temporary buffer
-                // (first frame of a batch that needs a bigger slot, or a frame that moves to the next batch)
-                uint8_t* dstp; bool to_tmp = false;
-                if (in_used + 12 + toRead <= s->in_cap) dstp = s->h_in + in_used;
-                else { carry.resize(12 + toRead); dstp = carry.data(); to_tmp = true; }
-                memcpy(dstp, hdr, 12);
-                if (pre) memcpy(dstp + 12, first + 12, pre);
-                const double tc0 = tr ? StageClock::now() : 0;
-                size_t g = 0; size_t e = read_some(E, rw, dstp + 12 + pre, toRead - pre, &g);
-                if (tr) rd_clk.cb += StageClock::now() - tc0;
-                if (e) { P.fail(e); failed = true; break; }
-                if (g != toRead - pre) { P.fail(E.data_error); failed = true; break; }
-                stat_in += g;
-                if (to_tmp) {
-                    if (n > 0) break;                                   // next batch starts with it
-                    if (!place_first(carry)) { failed = true; break; }
-                    carry.clear();
-                    continue;
-                }
-                uint64_t osz = 0; uint32_t nsq = 0;
-                uint32_t nblk_new = nblk; uint64_t scr_new = scr;
-                bool moves = false;                                     // does not fit behind the others: first frame of the next batch
-                if (!is_zstd) {
-                    if (!lz4f_out_size(dstp + 12, toRead, &osz)) { c->lib_errcode = ZMT_ST_BAD_HEADER; P.fail(E.library); failed = true; break; }
-                } else {
-                    // block table of this frame (descriptors are appended; dropped again if the frame moves to the next batch)
-                    uint64_t cs = 0;
-                    const double ts0 = tr ? StageClock::now() : 0;
-                    const int zr = zmt_zstd_scan_frame_host(dstp + 12, toRead, in_used + 12, n, s->h_blk, &nblk_new, s->blk_cap, &scr_new, &cs, &nsq);
-                    if (tr) rd_scan += StageClock::now() - ts0;
-                    if (zr == ZMT_ST_DST_SMALL) moves = true;
-                    else if (zr != ZMT_ST_OK) { c->lib_errcode = (size_t)zr; P.fail(zr == ZMT_ST_TRUNCATED || zr == ZMT_ST_TRAILING ? E.frame_decompress : E.library); failed = true; break; }
-                    else if (scr_new > s->scr_cap) moves = true;
-                    osz = cs;
-                }
-                if (!moves && osz > s->out_cap - out_used) moves = true;
-                if (moves) {
-                    carry.assign(dstp, dstp + 12 + toRead);
-                    if (n > 0) break;
-                    if (!place_first(carry)) { failed = true; break; }  // a single frame larger than the slot: grow the slot
-                    carry.clear();
-                    continue;
-                }
-                T.a[n] = in_used; T.d[n] = (uint32_t)toRead; T.b[n] = out_used;
-                if (is_zstd) { T.g[n] = nblk; T.f[n] = (nsq & 4u) ? ~0ull : osz; T.d[n] = nsq; nblk = nblk_new; scr = scr_new; }     // T.d = frame flags (sequential pass, checksum, no size)
-                in_used += 12 + toRead; out_used += osz; n++;
-            }
-            if (failed) break;
-            if (n == 0) break;
-            T.b[n] = out_used;
-            if (is_zstd) { T.g[n] = nblk; s->nblk = nblk; s->scratch_used = scr; }
-            s->n = n; s->in_used = in_used; s->out_used = (size_t)out_used;
-            { uint64_t ns = 0; for (uint32_t i = 0; i < n; i++) { const uint64_t nb = (T.b[i + 1] - T.b[i] + 65535) / 65536; ns += nb ? nb : 1; } s->nslots = (uint32_t)ns; }
-            {
-                std::lock_guard<std::mutex> g(P.mu);
-                c->insize += stat_in; c->frames += n;
-                s->state = 1; P.fill_seq++;
-            }
-            P.cv.notify_all();
-        }
-        if (tr) rd_total = StageClock::now() - t_start;
-        { std::lock_guard<std::mutex> g(P.mu); P.reader_done = true; }
-        P.cv.notify_all();
-    });
-
-    // ---- writer (pt_write, lz4-mt_decompress.c:165-187)
-    std::thread writer([&]() {
-        const ScopedAffinity bind(host_cpus);
-        const double t_start = tr ? StageClock::now() : 0;
-        for (;;) {
-            Slot* s;
-            {
-                std::unique_lock<std::mutex> lk(P.mu);
-                s = &P.slots[P.write_seq % N];
-                const double t0 = tr ? StageClock::now() : 0;
-                P.cv.wait(lk, [&] { return s->state == 2 || P.error || (P.reader_done && P.write_seq == P.fill_seq); });
-                if (tr) wr_clk.wait += StageClock::now() - t0;
-                if (P.error || s->state != 2) break;
-            }
-            cudaSetDevice(s->dev);
-            const double tg0 = tr ? StageClock::now() : 0;
-            if (cudaEventSynchronize(s->ev) != cudaSuccess) { c->lib_errcode = ZMT_ST_CUDA; P.fail(E.library); break; }
-            if (tr) wr_clk.gpu += StageClock::now() - tg0;
-            Tables T = tables_at(s->h_tab, s->tab_cap);
-            bool bad = false;
-            // The decoded bytes come over in pieces of a few MiB, one piece ahead of the one being written: what fn_write's
-            // memcpy reads was DMA-written moments ago and is still in the last-level cache, instead of a whole 64 MiB slot that
-            // was copied long before its first byte is used.
-            uint32_t issued = 0, ready = 0; int np_issued = 0, np_ready = 0;       // frames [0, issued) requested, [0, ready) landed
-            auto issue_piece = [&]() -> bool {
-                if (issued >= s->n) return true;
-                uint32_t j = issued; uint64_t lo = T.b[j], hi = lo;
-                while (j < s->n && hi - lo < piece_bytes) { hi = T.b[j] + T.c[j]; j++; }
-                if (hi > s->out_cap) hi = s->out_cap;
-                if (hi > lo && cudaMemcpyAsync(s->h_out + lo, s->d_out + lo, (size_t)(hi - lo), cudaMemcpyDeviceToHost, s->stream) != cudaSuccess) return false;
-                if (cudaEventRecord(s->evp[np_issued & 1], s->stream) != cudaSuccess) return false;
-                np_issued++; issued = j;
-                return true;
-            };
-            uint32_t piece_end[2] = { 0, 0 };
-            for (uint32_t i = 0; i < s->n; i++) {
-                const uint32_t st = T.e[i];
-                if (st != ZMT_ST_OK) {
-                    c->lib_errcode = st;
-                    P.fail((st == ZMT_ST_TRUNCATED || st == ZMT_ST_TRAILING) ? E.frame_decompress : E.library);
-                    bad = true; break;
-                }
-                if (piece_bytes && i >= ready) {
-                    bool okp = true;
-                    if (np_issued == np_ready) { okp = issue_piece(); piece_end[(np_issued - 1) & 1] = issued; }
-                    if (okp && issued < s->n && np_issued == np_ready + 1) { okp = issue_piece(); piece_end[(np_issued - 1) & 1] = issued; }   // one ahead
-                    if (okp) okp = cudaEventSynchronize(s->evp[np_ready & 1]) == cudaSuccess;
-                    if (!okp) { c->lib_errcode = ZMT_ST_CUDA; P.fail(E.library); bad = true; break; }
-                    ready = piece_end[np_ready & 1]; np_ready++;
-                }
-                GenBuffer b; b.buf = s->h_out + T.b[i]; b.size = (size_t)T.c[i]; b.allocated = b.size;
-                const double tc0 = tr ? StageClock::now() : 0;
-                int rv = rw->fn_write(rw->arg_write, &b);
-                if (tr) wr_clk.cb += StageClock::now() - tc0;
-                if (rv != 0) { P.fail(mt_error(E, rv)); bad = true; break; }
-                c->outsize += b.size; c->curframe++;
-            }
-            if (bad) break;
-            { std::lock_guard<std::mutex> g(P.mu); s->state = 0; P.write_seq++; }
-            P.cv.notify_all();
-        }
-    });
-
-    // ---- submit
-    for (;;) {
-        Slot* s;
-        {
-            std::unique_lock<std::mutex> lk(P.mu);
-            s = &P.slots[P.submit_seq % N];
-            P.cv.wait(lk, [&] { return s->state == 1 || P.error || (P.reader_done && P.submit_seq == P.fill_seq); });
-            if (P.error || s->state != 1) break;
-        }
-        cudaSetDevice(s->dev);
-        Tables Th = tables_at(s->h_tab, s->tab_cap), Td = tables_at(s->d_tab, s->tab_cap);
-        cudaError_t ce = cudaMemcpyAsync(s->d_in, s->h_in, s->in_used, cudaMemcpyHostToDevice, s->stream);
-        if (ce == cudaSuccess) ce = cudaMemcpyAsync(s->d_tab, s->h_tab, s->tab_bytes, cudaMemcpyHostToDevice, s->stream);
-        int st = ZMT_ST_CUDA;
-        if (ce == cudaSuccess && is_zstd && s->nblk) ce = cudaMemcpyAsync(s->d_blk, s->h_blk, (size_t)s->nblk * zmt_zstd_blk_desc_bytes(), cudaMemcpyHostToDevice, s->stream);
-        if (ce == cudaSuccess) st = is_zstd ? zmt_zstd_decompress_device(s->d_in, s->d_blk, s->nblk, Td.g, Td.f, Td.d, s->n, s->d_out, Td.b, Td.c, Td.e, s->d_work, s->stream)
-                                            : zmt_lz4_decompress_device(s->d_in, s->in_used, Td.a, Td.d, s->n, s->nslots, s->d_out, Td.b, Td.c, Td.e, s->d_work, s->stream);
-        if (s->dev >= 0 && s->dev < 64) g_dev_batches[s->dev]++;
-        if (st == ZMT_ST_OK) {
-            if (s->out_used && piece_bytes == 0) ce = cudaMemcpyAsync(s->h_out, s->d_out, s->out_used, cudaMemcpyDeviceToHost, s->stream);
-            if (ce == cudaSuccess) ce = cudaMemcpyAsync(Th.c, Td.c, (size_t)s->n * 8, cudaMemcpyDeviceToHost, s->stream);
-            if (ce == cudaSuccess) ce = cudaMemcpyAsync(Th.e, Td.e, (size_t)s->n * 4, cudaMemcpyDeviceToHost, s->stream);
-            if (ce == cudaSuccess) ce = cudaEventRecord(s->ev, s->stream);
-            if (ce != cudaSuccess) st = ZMT_ST_CUDA;
-        }
-        if (st != ZMT_ST_OK) { c->lib_errcode = (size_t)st; P.fail(E.library); break; }
-        { std::lock_guard<std::mutex> g(P.mu); s->state = 2; P.submit_seq++; }
-        P.cv.notify_all();
-    }
-    reader.join(); writer.join();
-    for (auto& s : P.slots) { if (s.ok) { cudaSetDevice(s.dev); cudaStreamSynchronize(s.stream); } }
-    if (tr)
-        fprintf(stderr, "[zstdmt_b200] decompress: reader total %.3fs cb %.3fs scan %.3fs wait %.3fs | writer gpu-wait %.3fs cb %.3fs wait %.3fs | slots %zu, batch %zu MiB\n",
-                rd_total, rd_clk.cb, rd_scan, rd_clk.wait, wr_clk.gpu, wr_clk.cb, wr_clk.wait, N, in_cap0 >> 20);
-    (void)wr_total;
-    return P.error;
+    const uint64_t piece_bytes = (uint64_t)env_size("ZSTDMT_B200_D2H_PIECE_MB", 2) << 20;      // 0: whole slot right after the kernels (measured 0 / 2 / 4 / 8 MiB: 12.8 / 15.1 / 14.3 / 12.8 GB/s)
+    return run_pipeline(c, P.slots.size(), [&](Slot& s, bool& last) { return reader.fill(s, last); },
+                        [&](Slot& s) { return decode_submit(c, s, piece_bytes); }, [&](Slot& s) { return decode_drain(c, rw, s, piece_bytes); });
 }
 
 // ------------------------------------------------------------------ context helpers
@@ -1142,8 +1110,6 @@ const char* status_string(size_t st)
 
 const char* error_string(bool lz4, size_t code, size_t lib_errcode)
 {
-    static const char* none = nullptr;
-    (void)none;
     const size_t neg = 0 - code;
     // the reference returns the codec library's own message whenever its global errcode is set
     // (lz4-mt_common.c:37-38); we own the status table instead of liblz4 / libzstd

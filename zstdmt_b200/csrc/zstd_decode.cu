@@ -1349,9 +1349,6 @@ static int zd_tables_init()
     return ZMT_ST_OK;
 }
 
-extern "C" int zmt_zstd_scan_frame_host2(const uint8_t* frame, size_t n, uint64_t base_off, uint32_t frame_idx, void* blocks_out, uint32_t* nblocks_io,
-                                         uint32_t max_blocks, uint64_t* scratch_used, uint64_t* content_size, uint32_t* needs_seq, size_t* consumed);
-
 static inline uint32_t h_rd32(const uint8_t* p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24); }
 
 // Walk one zstd frame on the host (frame header + 3-byte block headers + the two section headers of every
